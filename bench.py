@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this back end
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle/_ref)
+    python bench.py ... --dump-outputs DIR                   # also write a fixed sample of the timed path's frames
 
 Headline workload (default): BASELINE.json configs[4] -- the batch of independent viewpoints of the
 TEXTURED ~2.5k-triangle mesh (nearest texel, gamma-2 pipeline, Gouraud) at 1920x1080 colour+z,
@@ -161,6 +162,34 @@ class ViewScene:
                 r.set_target(f)
                 for kw in self.overlays:
                     r.rectangle(**kw)
+
+
+DUMP_FRAMES, DUMP_PIXELS, DUMP_CROP = 512, 1 << 21, 512
+
+
+def dump_outputs(out_dir, prefix, read_frame, n_frames, w, h):
+    """--dump-outputs: the frames the timed path left behind after its last step, as float32 .npy files, so that
+    two builds run with the same arguments (hence the same inputs) can be compared output for output.  The sample
+    is fixed (seed 0): at most DUMP_FRAMES of the n_frames frames, the same DUMP_PIXELS // frames pixels of each,
+    and the whole DUMP_CROP x DUMP_CROP centre of the last of those frames.  A colour pixel is split into its four bytes
+    (memory order B, G, R, X), so a one-level difference in any channel shows; depth is written as stored.
+    At most 2M x 20 B + 512^2 x 20 B = 47 MB.  read_frame(i) returns frame i's (colour u32, depth f32) planes."""
+    rng = np.random.default_rng(0)
+    frames = np.arange(n_frames) if n_frames <= DUMP_FRAMES else np.sort(rng.choice(n_frames, DUMP_FRAMES, replace=False))
+    pix = np.sort(rng.choice(w * h, min(w * h, DUMP_PIXELS // len(frames)), replace=False))
+    col_s = np.empty((len(frames), len(pix), 4), np.float32)
+    z_s = np.empty((len(frames), len(pix)), np.float32)
+    for j, f in enumerate(frames):
+        col, z = read_frame(int(f))
+        col_s[j] = col.reshape(-1)[pix].view(np.uint8).reshape(-1, 4)
+        z_s[j] = z.reshape(-1)[pix]
+    y0, x0 = max(0, (h - DUMP_CROP) // 2), max(0, (w - DUMP_CROP) // 2)
+    col_c = np.ascontiguousarray(col[y0:y0 + DUMP_CROP, x0:x0 + DUMP_CROP])
+    z_c = z[y0:y0 + DUMP_CROP, x0:x0 + DUMP_CROP]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("color_sample", col_s), ("depth_sample", z_s),
+                    ("color_crop", col_c.view(np.uint8).reshape(*col_c.shape, 4)), ("depth_crop", z_c)):
+        np.save(os.path.join(out_dir, f"{prefix}_{name}.npy"), a.astype(np.float32))
 
 
 def oracle_kind():
@@ -377,9 +406,10 @@ class Env:
         return self.torch.cuda.Event(enable_timing=True), self.torch.cuda.Event(enable_timing=True)
 
 
-def measure_views(env, name, views, steps, warmup, e2e_steps, with_e2e):
+def measure_views(env, name, views, steps, warmup, e2e_steps, with_e2e, dump=None):
     """One frame-parallel workload on this rank's GPU: device-resident throughput (replay of one
-    B-view flush), per-stage times, parity of frames rendered by the timed path, optional e2e."""
+    B-view flush), per-stage times, parity of frames rendered by the timed path, optional e2e;
+    dump: directory for dump_outputs() of the frames of the last timed replay."""
     torch = env.torch
     s = WORKLOADS[name]
     w, h, B = s["w"], s["h"], views
@@ -425,6 +455,10 @@ def measure_views(env, name, views, steps, warmup, e2e_steps, with_e2e):
     # parity of what the TIMED path left in the frames: first, middle and last view of this rank
     pairs = sorted({(0, view0), (B // 2, view0 + B // 2), (B - 1, view0 + B - 1)})
     checked = check_view_frames(r, scene, pairs)
+    if dump:
+        cbuf, zbuf = np.empty((h, w), np.uint32), np.empty((h, w), np.float32)
+        dump_outputs(dump, name + (f"_rank{env.rank}" if env.world > 1 else ""),
+                     lambda f: r.end_frame(f, color_out=cbuf, z_out=zbuf), B, w, h)
     # untimed extra pass with the replay pipelining off: per-stage times in isolation (in the timed
     # region the pre-raster stages of later replays overlap the raster kernel, so their event
     # intervals include the wait for free SMs and the stages no longer add up to the step)
@@ -605,11 +639,12 @@ def run_fill_reference(args, rank, world):
         flush=True)
 
 
-def measure_fill(env, name, n_override, steps, warmup, e2e_steps, gather, with_e2e, band_frames=2):
+def measure_fill(env, name, n_override, steps, warmup, e2e_steps, gather, with_e2e, band_frames=2, dump=None):
     """cfg 4 on this process group: one frame of 1M small triangles; N>1 splits the screen into
     tile-aligned bands (every rank runs setup over all triangles, bins and rasterises its band) and
     assembles the frame in rank 0's HBM.  Parity: the assembled planes == rank 0's own whole-frame
-    render, and (N=1, full size) == the reference oracle."""
+    render, and (N=1, full size) == the reference oracle.  dump: directory for dump_outputs() of the
+    frame in rank 0's HBM after the timed steps."""
     torch, multigpu = env.torch, env.multigpu
     f = FILL[name]
     w, h, n = f["w"], f["h"], n_override or f["n"]
@@ -702,22 +737,23 @@ def measure_fill(env, name, n_override, steps, warmup, e2e_steps, gather, with_e
         env.stream.synchronize()
         s2.synchronize()
         env.barrier()
-        steps2 = steps + (steps & 1)
         env.clocks.start()
         e0.record(env.stream)
         s2.wait_stream(env.stream)
-        run_alternating(steps2)
+        run_alternating(steps)
         env.stream.wait_stream(s2)
         e1.record(env.stream)
         env.barrier()
         env.clocks.pause()
-        ms_step = env.max_over_ranks(e0.elapsed_time(e1)) / steps2
+        ms_step = env.max_over_ranks(e0.elapsed_time(e1)) / steps
         env.launches += r2.stats()["kernelLaunches"]
 
     # ---- parity of the frame(s) the timed steps left in rank 0's HBM ---------------------------
     parity = []
     if rank == 0:
         col, z = r.end_frame(0)
+        if dump:
+            dump_outputs(dump, name, lambda f: (col, z), 1, w, h)
         if r2 is not None:
             col_b, z_b = r2.end_frame(0)
             if not (np.array_equal(col, col_b) and np.array_equal(z.view(np.uint32), z_b.view(np.uint32))):
@@ -813,9 +849,10 @@ def run_gpu_arm(args, rank, world, local_rank):
         bind_to_gpu_numa_node(local_rank)
     e2e_steps = max(2, min(args.steps, args.e2e_steps))
     if main_is_fill:
-        main = measure_fill(env, args.workload, args.triangles, args.steps, args.warmup, e2e_steps, args.gather, True, args.band_frames)
+        main = measure_fill(env, args.workload, args.triangles, args.steps, args.warmup, e2e_steps, args.gather, True, args.band_frames,
+                            args.dump_outputs)
     else:
-        main = measure_views(env, args.workload, views, args.steps, args.warmup, e2e_steps, True)
+        main = measure_views(env, args.workload, views, args.steps, args.warmup, e2e_steps, True, args.dump_outputs)
     others = []
     if not args.no_others:
         o_steps = max(5, min(args.steps, 20))
@@ -886,7 +923,14 @@ def main():
                          "1 = one target, the barrier in line (always measured and reported as well)")
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="fill4k, N>1: how the bands reach rank 0 (peer-memory write-back or NCCL send/recv)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of the frames the timed path rendered in its last step "
+                         "to DIR/<name>.npy (float32, under 64 MB in all); see dump_outputs()")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the frames of the B200 arm's timed path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

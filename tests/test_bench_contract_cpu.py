@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -45,6 +48,38 @@ def test_raster_stage_split_labels():
     assert bench.kernel_split((4.0, 0.0), 2, 0, True) == {"raster_tex_kernel": 2.0}
     assert bench.kernel_split((4.0, 0.0), 0, 0, False) == {"raster_kernel": 4.0}
     assert bench.stage_label(2, True).startswith("raster_opaque_kernel<true>") and bench.stage_label(0, False) == "raster_kernel"
+
+
+@pytest.mark.parametrize("n_frames,w,h", [(512, 1920, 1080), (1000, 64, 48), (1, 3840, 2160)])
+def test_dump_outputs_is_a_fixed_bounded_sample(tmp_path, n_frames, w, h):
+    """--dump-outputs: float32 files under 64 MB in all, the same sample on every run, and every sampled value is
+    the pixel it claims to be (frame f's pixel i holds colour f * w * h + i and depth i, so both can be decoded)."""
+    sys.path.insert(0, ROOT)
+    import bench
+    idx = np.arange(w * h, dtype=np.uint32).reshape(h, w)
+
+    def read_frame(f):
+        return idx + np.uint32(f * w * h), idx.astype(np.float32)
+
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), "wl", read_frame, n_frames, w, h)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["wl_color_crop.npy", "wl_color_sample.npy", "wl_depth_crop.npy", "wl_depth_sample.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 << 20
+    out = {}
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+        out[n[3:-4]] = a
+    col = out["color_sample"].astype(np.uint8).view(np.uint32)[..., 0].astype(np.int64)
+    frames, pix = np.divmod(col, w * h)
+    assert np.array_equal(pix, out["depth_sample"].astype(np.int64))
+    assert np.all(pix == pix[0]) and np.all(np.diff(pix[0]) > 0)  # the same pixels of every frame
+    assert np.all(frames == frames[:, :1]) and np.all(np.diff(frames[:, 0]) > 0) and frames[-1, 0] < n_frames
+    assert len(frames) == min(n_frames, bench.DUMP_FRAMES)
+    crop = out["color_crop"].astype(np.uint8).view(np.uint32)[..., 0].astype(np.int64)
+    assert crop.shape == (min(h, bench.DUMP_CROP), min(w, bench.DUMP_CROP))
+    assert np.all(crop // (w * h) == frames[-1, 0]) and np.array_equal(crop % (w * h), out["depth_crop"].astype(np.int64))
 
 
 def test_gpu_arm_fails_loudly_without_a_device(built):
