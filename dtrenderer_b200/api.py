@@ -94,6 +94,9 @@ SYMBOLS = [
     ("dtr_b200_set_output_planes", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     ("dtr_b200_enable_peer_access", C.c_int, [C.c_void_p, C.c_int]),
     ("dtr_b200_frame_device_ptrs", C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
+    ("dtr_b200_set_id_output", C.c_int, [C.c_void_p, C.c_int]),
+    ("dtr_b200_read_ids", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    ("dtr_b200_frame_id_ptr", C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
     ("dtr_b200_get_stats", C.c_int, [C.c_void_p, C.POINTER(Stats)]),
     ("dtr_b200_reset_stats", C.c_int, [C.c_void_p]),
     ("dtr_b200_last_pass_deferred", C.c_int, [C.c_void_p]),
@@ -397,6 +400,24 @@ class Renderer:
         c, z = C.c_void_p(), C.c_void_p()
         self._ck(self.lib.dtr_b200_frame_device_ptrs(self.ctx, frame, C.byref(c), C.byref(z)))
         return c.value, z.value
+
+    # ---- triangle id planes (see dtr_b200_set_id_output) ----------------------------------------
+    def set_id_output(self, on=True):
+        """Keep a u32 id plane per frame: 1 + the frame position of the triangle whose fragment last wrote
+        a pixel's depth since the frame's begin_frame, 0 where none did (for one mesh call: face index + 1)."""
+        self._ck(self.lib.dtr_b200_set_id_output(self.ctx, 1 if on else 0))
+
+    def read_ids(self, first=0, n=1):
+        """Flush and read the id planes of frames [first, first + n): u32[n, H, W]."""
+        out = np.empty((n, self.height, self.width), np.uint32)
+        self._ck(self.lib.dtr_b200_read_ids(self.ctx, first, n, out.ctypes.data_as(C.c_void_p)))
+        return out
+
+    def frame_id_ptr(self, frame=0):
+        """Device address of a frame's id plane (u32[H*W])."""
+        p = C.c_void_p()
+        self._ck(self.lib.dtr_b200_frame_id_ptr(self.ctx, frame, C.byref(p)))
+        return p.value
 
     def stats(self):
         s = Stats()

@@ -63,6 +63,7 @@ struct FrameHost
 	uint32_t pendingInit = 0; // FrameInit bits to apply at the next flush
 	uint32_t clearPacked = 0;
 	uint32_t recorded    = 0; // items recorded for this frame since the last flush
+	uint32_t triangles   = 0; // triangles submitted since the frame's last dtr_b200_begin_frame: the next one's id is this + 1
 };
 
 } // namespace
@@ -95,6 +96,7 @@ struct dtr_b200_ctx
 	// write straight into the gathering rank's frames over NVLink, dtr_b200_open_peer_frames)
 	uint32_t    *outColor = nullptr;
 	float       *outDepth = nullptr;
+	uint32_t    *dIds = nullptr; // triangle id planes u32[F][H][W] (dtr_b200_set_id_output), always this context's own; null: off
 	void        *ipcColor = nullptr, *ipcDepth = nullptr; // mappings opened from IPC handles
 	Geometry     geom{};
 	int          target = 0;
@@ -130,6 +132,7 @@ struct dtr_b200_ctx
 	struct PipeSet
 	{
 		DevBuf              prims, bounds, primZ, tileCount, tileOffset, order, lists, listBounds, listZ, segRel;
+		DevBuf              primId; // ids on: per primitive, its triangle id (setup_kernel)
 		unsigned long long *counters = nullptr; // [1] list total, [3] work counter, [4] busy tiles
 		cudaEvent_t         preDone = nullptr, rasterDone = nullptr;
 		bool                rasterPending = false; // rasterDone has been recorded: the set may still be read
@@ -252,6 +255,12 @@ RecItem &new_item(dtr_b200_ctx *c, uint32_t type, uint32_t frame, uint32_t count
 	r.frame      = frame;
 	r.order      = (uint32_t)c->rec.size() - 1;
 	c->frames[frame].recorded++;
+	if (type != ITEM_RAW)
+	{
+		// triangles are numbered per frame in submission order, across flushes (triangle id planes)
+		r.item.triBase = c->frames[frame].triangles;
+		c->frames[frame].triangles += count;
+	}
 	return r;
 }
 
@@ -353,6 +362,7 @@ int run_pipeline(dtr_b200_ctx *c, uint32_t numActive, uint32_t numItems, uint32_
 	if ((rc = ensure_dev(c, S.prims, sizeof(PrimRecord) * (size_t)std::max(numPrims, 1u)))) return rc;
 	if ((rc = ensure_dev(c, S.bounds, sizeof(PrimBounds) * (size_t)std::max(numPrims, 1u)))) return rc;
 	if ((rc = ensure_dev(c, S.primZ, sizeof(int32_t) * (size_t)std::max(numPrims, 1u)))) return rc;
+	if (c->dIds && (rc = ensure_dev(c, S.primId, sizeof(uint32_t) * (size_t)std::max(numPrims, 1u)))) return rc;
 	uint32_t *dSegCount  = (uint32_t *)S.tileCount.p;
 	uint32_t *dTileCount = g.segs > 1 ? dSegCount + numSeg : dSegCount; // with one segment they are the same thing
 
@@ -376,6 +386,7 @@ int run_pipeline(dtr_b200_ctx *c, uint32_t numActive, uint32_t numItems, uint32_
 		SP.frames      = dFrames;
 		SP.textures    = (const TexDesc *)c->dTextures.p;
 		SP.g           = g;
+		SP.primId      = c->dIds ? (uint32_t *)S.primId.p : nullptr;
 		launch_setup(SP, pre);
 		c->launches++;
 	}
@@ -470,6 +481,8 @@ int run_pipeline(dtr_b200_ctx *c, uint32_t numActive, uint32_t numItems, uint32_
 	R.numTiles       = 0;
 	R.smallTilesMin  = 0;
 	R.g          = g;
+	R.ids        = c->dIds; // the IDS variants of the stage's kernels, or (null) the ones without id logic
+	R.primId     = c->dIds ? (const uint32_t *)S.primId.p : nullptr;
 	if ((rc = mark(c, c->stream))) return rc;
 	if (c->last.deferred)
 	{
@@ -716,7 +729,7 @@ void dtr_b200_destroy(dtr_b200_ctx *c)
 	std::vector<DevBuf *> bufs = {&c->dTextures, &c->dCmd, &c->dPayload};
 	for (auto &ps : c->sets)
 	{
-		for (DevBuf *b : {&ps.prims, &ps.bounds, &ps.primZ, &ps.tileCount, &ps.tileOffset, &ps.order, &ps.lists, &ps.listBounds, &ps.listZ, &ps.segRel}) bufs.push_back(b);
+		for (DevBuf *b : {&ps.prims, &ps.bounds, &ps.primZ, &ps.tileCount, &ps.tileOffset, &ps.order, &ps.lists, &ps.listBounds, &ps.listZ, &ps.segRel, &ps.primId}) bufs.push_back(b);
 		cudaFree(ps.counters);
 		if (ps.preDone) cudaEventDestroy(ps.preDone);
 		if (ps.rasterDone) cudaEventDestroy(ps.rasterDone);
@@ -728,6 +741,7 @@ void dtr_b200_destroy(dtr_b200_ctx *c)
 	if (c->ipcDepth) cudaIpcCloseMemHandle(c->ipcDepth);
 	cudaFree(c->dColor);
 	cudaFree(c->dDepth);
+	cudaFree(c->dIds);
 	cudaFree(c->dSetPixels);
 	if (c->payload) cudaFreeHost(c->payload);
 	if (c->staging) cudaFreeHost(c->staging);
@@ -1001,9 +1015,15 @@ int dtr_b200_begin_frame(dtr_b200_ctx *c, int frame, const uint32_t *hostColor, 
 	// a dtr_b200_clear recorded as the frame's on-chip colour init stays pending (the reference's
 	// Clear writes the colour buffer, the frame start only resets depth) unless colour is uploaded now
 	fh.pendingInit &= FI_COLOR_CLEAR;
+	fh.triangles = 0;
 	// an asynchronous readback of this frame may still be in flight on the copy stream
 	if ((hostZ || hostColor) && frame >= c->readLo && frame < c->readHi) CU(cudaStreamWaitEvent(c->stream, c->copyDone, 0));
-	if (hostZ) CU(cudaMemcpyAsync(c->outDepth + plane * frame, hostZ, plane * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+	if (hostZ)
+	{
+		CU(cudaMemcpyAsync(c->outDepth + plane * frame, hostZ, plane * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+		// uploaded depth was written by no triangle of this frame (a reset depth zeroes the ids on chip, with FI_Z_RESET)
+		if (c->dIds) CU(cudaMemsetAsync(c->dIds + plane * frame, 0, plane * sizeof(uint32_t), c->stream));
+	}
 	else fh.pendingInit |= FI_Z_RESET;
 	if (hostColor)
 	{
@@ -1344,6 +1364,62 @@ int dtr_b200_frame_device_ptrs(dtr_b200_ctx *c, int frame, void **color, void **
 	size_t plane = (size_t)c->width * c->height;
 	if (color) *color = c->outColor + plane * frame;
 	if (z) *z = c->outDepth + plane * frame;
+	return DTR_B200_OK;
+}
+
+int dtr_b200_set_id_output(dtr_b200_ctx *c, int enable)
+{
+	if (!c) return DTR_B200_ERR_ARG;
+	CU(cudaSetDevice(c->device));
+	if ((enable != 0) == (c->dIds != nullptr)) return DTR_B200_OK;
+	// (enqueued passes may still use the buffers; draw calls recorded but not yet flushed run with the new setting)
+	CU(cudaStreamSynchronize(c->preStream));
+	CU(cudaStreamSynchronize(c->stream));
+	if (!enable)
+	{
+		CU(cudaFree(c->dIds));
+		c->dIds = nullptr;
+		for (auto &ps : c->sets)
+		{
+			CU(cudaFree(ps.primId.p));
+			ps.primId = DevBuf();
+		}
+		return DTR_B200_OK;
+	}
+	const size_t bytes = (size_t)c->width * c->height * c->numFrames * sizeof(uint32_t);
+	uint32_t    *d     = nullptr;
+	const cudaError_t e = cudaMalloc((void **)&d, bytes);
+	if (e == cudaErrorMemoryAllocation)
+	{
+		cudaGetLastError(); // (not sticky: clear it)
+		return fail(c, DTR_B200_ERR_NOMEM, "allocating the triangle id planes", e);
+	}
+	if (e != cudaSuccess) return fail(c, DTR_B200_ERR_CUDA, "allocating the triangle id planes", e);
+	c->dIds = d;
+	CU(cudaMemsetAsync(c->dIds, 0, bytes, c->stream));
+	return DTR_B200_OK;
+}
+
+int dtr_b200_read_ids(dtr_b200_ctx *c, int first, int n, uint32_t *hostIds)
+{
+	if (!c) return DTR_B200_ERR_ARG;
+	if (!c->dIds) return fail(c, DTR_B200_ERR_ARG, "triangle id output is off (dtr_b200_set_id_output)");
+	if (!hostIds || n <= 0 || !valid_frame(c, first) || !valid_frame(c, first + n - 1)) return fail(c, DTR_B200_ERR_ARG, "frame range out of bounds");
+	CU(cudaSetDevice(c->device));
+	int rc = do_flush(c);
+	if (rc) return rc;
+	const size_t plane = (size_t)c->width * c->height;
+	CU(cudaMemcpyAsync(hostIds, c->dIds + plane * first, plane * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+	CU(cudaStreamSynchronize(c->stream));
+	return DTR_B200_OK;
+}
+
+int dtr_b200_frame_id_ptr(dtr_b200_ctx *c, int frame, void **ids)
+{
+	if (!c || !ids) return DTR_B200_ERR_ARG;
+	if (!c->dIds) return fail(c, DTR_B200_ERR_ARG, "triangle id output is off (dtr_b200_set_id_output)");
+	if (!valid_frame(c, frame)) return fail(c, DTR_B200_ERR_ARG, "frame out of range");
+	*ids = c->dIds + (size_t)c->width * c->height * frame;
 	return DTR_B200_OK;
 }
 

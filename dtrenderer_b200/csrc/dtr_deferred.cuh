@@ -26,6 +26,9 @@
 //                       second pass over the busy tiles and a second kernel.  (The first form of the
 //                       stage; kept selectable: it is the measured baseline of the one-kernel form.)
 //
+// Triangle id planes (RasterParams::ids): the IDS instantiations keep an id tile per warp beside the tag tile
+// and write it back with the region; the ids are final then, so resolve_kernel needs no id logic.
+//
 // Inexact triangles (sequential fp32 accumulation, see raster_tri_replay) cannot be re-evaluated per
 // pixel without their accumulation order; their fragments are shaded at once in the walk (a
 // __noinline__ call on a path that ~2 % of mesh triangles take) and stored as finished colours.
@@ -40,6 +43,7 @@ struct VisSmem
 	uint4    sub[32];           // current triangle, per sub-block: {E1,E2,E3 at its origin as fp32 (exact), in-bbox pixel mask}
 };
 constexpr int      VIS_CTAS_PER_SM = 6;
+constexpr int      VIS_IDS_CTAS_PER_SM = 4; // the id-plane variants: what their shared memory (VisSmem + IdSmem per warp) allows
 #ifndef DTR_VIS_LANE_COUNT
 #define DTR_VIS_LANE_COUNT 1 // SetPixel calls counted per lane (no vote in the coverage step), summed once per warp
 #endif
@@ -220,8 +224,9 @@ __device__ __forceinline__ void shade_opaque_wide(const uint4 *const (&rec)[N], 
 // One region of the visibility pass (see process_region for the walk; only the differences are commented).
 // FUSED: the pending pixels of the finished region are shaded HERE, from shared memory, before the region
 // is written back (see raster_visres_kernel); the region then leaves the SM with finished colours only.
-template <bool FUSED>
-__device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSmem &W, const int lane, const RegionJob &J,
+// IDS: the triangle ids as well, in I->t, set where a fragment sets its depth (and its tag, or its colour).
+template <bool FUSED, bool IDS = false>
+__device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSmem &W, IdSmem *I, const int lane, const RegionJob &J,
                                                    uint32_t &shaded, uint32_t &nextItem)
 {
 	const uint32_t FULL = 0xffffffffu, ltMask = (1u << lane) - 1u;
@@ -232,6 +237,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 	const float    zInit = -FLT_MAX;
 	const int      vr = (lane >> 1) & 3, vx = (lane >> 3) * SUB_W + (lane & 1) * 4;
 	const int      vsi = lane * 4;
+	uint32_t *const gI = IDS ? P.ids + (J.gZ - P.depth) : nullptr; // the region's frame in the id planes
 
 	if (J.count == 0)
 	{
@@ -249,6 +255,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 					const size_t gi = (size_t)y * width + x;
 					if (J.genC) frame_store(reinterpret_cast<uint4 *>(J.gC + gi), c4);
 					if (J.genZ) frame_store(reinterpret_cast<float4 *>(J.gZ + gi), z4);
+					if (IDS && J.genZ) frame_store(reinterpret_cast<uint4 *>(gI + gi), make_uint4(0u, 0u, 0u, 0u));
 				}
 			}
 		}
@@ -262,6 +269,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 					const size_t gi = (size_t)y * width + x;
 					if (J.genC) J.gC[gi] = J.clearPacked;
 					if (J.genZ) J.gZ[gi] = zInit;
+					if (IDS && J.genZ) gI[gi] = 0u;
 				}
 			}
 		}
@@ -288,6 +296,20 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			sc += SUBS_X * 32;
 			sz += SUBS_X * 32;
 		}
+		if (IDS)
+		{
+			const uint4 *pi = reinterpret_cast<const uint4 *>(gI + vOff);
+			uint32_t    *si = I->t + vsi;
+#pragma unroll 4
+			for (int i = 0; i < subsY; i++)
+			{
+				uint4 i4 = make_uint4(0u, 0u, 0u, 0u);
+				if (!J.genZ && i < vRows) i4 = *pi;
+				*reinterpret_cast<uint4 *>(si) = i4;
+				pi += width;
+				si += SUBS_X * 32;
+			}
+		}
 	}
 	else
 	{
@@ -299,6 +321,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			const int    si = pix_index((ry >> 2) * SUBS_X + (rx >> 3), ((ry & 3) << 3) + (rx & 7));
 			W.c[si] = J.clearPacked;
 			W.z[si] = (J.genZ || !in) ? zInit : J.gZ[gi];
+			if (IDS) I->t[si] = (J.genZ || !in) ? 0u : gI[gi];
 		}
 	}
 	__syncwarp();
@@ -310,12 +333,13 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 	const uint32_t laneBit = 1u << lane;
 	const uint32_t zAddrLane = (uint32_t)__cvta_generic_to_shared(W.z + lane);
 	const uint32_t cAddrLane = (uint32_t)__cvta_generic_to_shared(W.c + lane);
+	const uint32_t iAddrLane = IDS ? (uint32_t)__cvta_generic_to_shared(I->t + lane) : 0u;
 	const int      lx = lane & 7, ly = lane >> 3;
 	const int      sxo = (lane & 3) * SUB_W, syo = (lane >> 2) * SUB_H;
 
 	// exact triangle: classification and table as in raster_tri; a passing fragment writes its depth
 	// and its primitive's tag, nothing else
-	auto raster_tri = [&](const uint4 g0, const uint4 g1, const uint4 g2, const uint4 g3, const uint4 g4) {
+	auto raster_tri = [&](const uint4 g0, const uint4 g1, const uint4 g2, const uint4 g3, const uint4 g4, const uint32_t id) {
 		const int      x0 = g0.w & 0xFF, y0 = (g0.w >> 8) & 0xFF, x1 = (g0.w >> 16) & 0xFF, y1 = g0.w >> 24;
 		const float4   zp  = u2f4(g4); // 1/area, z1, z2-z1, z3-z1
 		const uint32_t tag = VIS_PENDING | g2.w;
@@ -360,6 +384,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			             :
 			             : "r"((uint32_t)pass), "r"(za), "f"(z), "r"(ca), "r"(tag)
 			             : "memory");
+			if (IDS) asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %0, 0;\n\t@q st.shared.u32 [%1], %2;\n\t}" : : "r"((uint32_t)pass), "r"(iAddrLane + (s << 7)), "r"(id) : "memory");
 #if DTR_VIS_LANE_COUNT
 			passes += pass ? 1u : 0u;
 #else
@@ -376,7 +401,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 	// sub-block layout falls on 32 different banks.  The edge functions are carried as fp32 and stepped
 	// by +8 dx / +4 dy: every value is an integer below 2^24 (the PF_EXACT bound covers the bbox grown by
 	// one window), so the sums are exact and the bits equal those of the table path.
-	auto raster_tri_small = [&](const uint4 g0, const uint4 g1, const uint4 g2, const uint4 g4, const int nwx, const int nwy) {
+	auto raster_tri_small = [&](const uint4 g0, const uint4 g1, const uint4 g2, const uint4 g4, const int nwx, const int nwy, const uint32_t id) {
 		const int      x0 = g0.w & 0xFF, y0 = (g0.w >> 8) & 0xFF, x1 = (g0.w >> 16) & 0xFF, y1 = g0.w >> 24;
 		const float4   zp  = u2f4(g4); // 1/area, z1, z2-z1, z3-z1
 		const uint32_t tag = VIS_PENDING | g2.w;
@@ -411,6 +436,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 				             :
 				             : "r"((uint32_t)pass), "r"(za), "f"(z), "r"(za - (uint32_t)(sizeof(uint32_t) * REGION_WORDS)), "r"(tag)
 				             : "memory");
+				if (IDS) asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %0, 0;\n\t@q st.shared.u32 [%1], %2;\n\t}" : : "r"((uint32_t)pass), "r"(iAddrLane + (za - zAddrLane)), "r"(id) : "memory");
 				passes += pass ? 1u : 0u;
 				e1 += sx1; e2 += sx2; e3 += sx3;
 				za += 32u * 4u; // the same pixel of the sub-block to the right
@@ -424,7 +450,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 #endif
 
 	// inexact triangle: the row-shared replay of raster_tri_replay; fragments are shaded at once
-	auto raster_tri_replay = [&](const uint32_t pidx, const uint4 g0, const uint4 g1, const uint4 g2, const uint4 g4) {
+	auto raster_tri_replay = [&](const uint32_t pidx, const uint4 g0, const uint4 g1, const uint4 g2, const uint4 g4, const uint32_t id) {
 		const int    x0 = g0.w & 0xFF, y0 = (g0.w >> 8) & 0xFF, x1 = (g0.w >> 16) & 0xFF, y1 = g0.w >> 24;
 		const float4 zp = u2f4(g4);
 		const float  fdx1 = __uint_as_float(g1.x), fdx2 = __uint_as_float(g1.y), fdx3 = __uint_as_float(g1.z);
@@ -459,6 +485,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			{
 				W.z[si] = z;
 				W.c[si] = shade_opaque_now(P.prims + pidx, e1, e2, e3);
+				if (IDS) I->t[si] = id;
 #if DTR_VIS_LANE_COUNT
 				passes++;
 #endif
@@ -584,22 +611,24 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 				    exact ? 0u : pidx);
 #endif
 				W.geo[r * 5 + 4] = q4;
+				if (IDS) I->geo[r] = __ldg(P.primId + pidx);
 			}
 			__syncwarp();
 			for (int r = 0; r < ng; r++)
 			{
-				const uint4 g0r = W.geo[r * 5], g1 = W.geo[r * 5 + 1], g2 = W.geo[r * 5 + 2], g3 = W.geo[r * 5 + 3], g4 = W.geo[r * 5 + 4];
+				const uint4    g0r = W.geo[r * 5], g1 = W.geo[r * 5 + 1], g2 = W.geo[r * 5 + 2], g3 = W.geo[r * 5 + 3], g4 = W.geo[r * 5 + 4];
+				const uint32_t id = IDS ? I->geo[r] : 0u;
 				if (g1.w & PF_EXACT)
 				{
 #if DTR_VIS_SMALL_WINDOWS
 					const int bw = (int)((g0r.w >> 16) & 0xFF) - (int)(g0r.w & 0xFF), bh = (int)(g0r.w >> 24) - (int)((g0r.w >> 8) & 0xFF);
 					const int nwx = (bw + SUB_W - 1) / SUB_W, nwy = (bh + SUB_H - 1) / SUB_H;
-					if (nwx * nwy <= DTR_VIS_SMALL_WINDOWS) raster_tri_small(g0r, g1, g2, g4, nwx, nwy);
+					if (nwx * nwy <= DTR_VIS_SMALL_WINDOWS) raster_tri_small(g0r, g1, g2, g4, nwx, nwy, id);
 					else
 #endif
-						raster_tri(g0r, g1, g2, g3, g4);
+						raster_tri(g0r, g1, g2, g3, g4, id);
 				}
-				else raster_tri_replay(g3.w, g0r, g1, g2, g4);
+				else raster_tri_replay(g3.w, g0r, g1, g2, g4, id);
 			}
 			__syncwarp();
 		}
@@ -682,6 +711,19 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			sc += SUBS_X * 32;
 			sz += SUBS_X * 32;
 		}
+		if (IDS)
+		{
+			uint4          *pi = reinterpret_cast<uint4 *>(gI + vOff);
+			const uint32_t *si = I->t + vsi;
+			const int       n  = min(subsY, vRows);
+#pragma unroll 4
+			for (int i = 0; i < n; i++)
+			{
+				frame_store(pi, *reinterpret_cast<const uint4 *>(si));
+				pi += width;
+				si += SUBS_X * 32;
+			}
+		}
 	}
 	else
 	{
@@ -694,6 +736,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 				const int    si = pix_index((ry >> 2) * SUBS_X + (rx >> 3), ((ry & 3) << 3) + (rx & 7));
 				J.gC[gi] = W.c[si];
 				J.gZ[gi] = W.z[si];
+				if (IDS) gI[gi] = I->t[si];
 			}
 		}
 	}
@@ -702,11 +745,14 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 
 // the persistent item loop of raster_body, for the visibility pass
 // (the kernels are instantiations of one __global__ template rather than wrappers around a device function: the
-// two-kernel form keeps exactly the machine code it was measured with)
-template <bool FUSED>
-__global__ void __launch_bounds__(128, FUSED ? DTR_FUSED_CTAS : VIS_CTAS_PER_SM) raster_opaque_kernel(RasterParams P)
+// two-kernel form keeps exactly the machine code it was measured with).  IDS: the variant that also keeps the
+// triangle id planes (RasterParams::ids), with 16 KB more shared memory per CTA.
+template <bool FUSED, bool IDS = false>
+__global__ void __launch_bounds__(128, IDS ? VIS_IDS_CTAS_PER_SM : (FUSED ? DTR_FUSED_CTAS : VIS_CTAS_PER_SM)) raster_opaque_kernel(RasterParams P)
 {
 	__shared__ __align__(16) VisSmem sW[4];
+	IdSmem *I = nullptr;
+	if constexpr (IDS) I = id_smem();
 	const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 	for (size_t i = (size_t)blockIdx.x * 128 + tid; i < P.zeroWords; i += (size_t)gridDim.x * 128) P.zeroBase[i] = 0u;
 
@@ -774,8 +820,8 @@ __global__ void __launch_bounds__(128, FUSED ? DTR_FUSED_CTAS : VIS_CTAS_PER_SM)
 				{
 					const bool genZ = (e1[k].y & FI_Z_RESET) != 0, genC = (e1[k].y & FI_COLOR_CLEAR) != 0;
 					if (genZ || genC)
-						stream_empty_tile(P, (int)(e1[k].z & 0xFFFFu), (int)(e1[k].z >> 16), P.color + plane * fr[k], P.depth + plane * fr[k], genC,
-						                  genZ, e1[k].x, lane);
+						stream_empty_tile<IDS>(P, (int)(e1[k].z & 0xFFFFu), (int)(e1[k].z >> 16), P.color + plane * fr[k], P.depth + plane * fr[k],
+						                       IDS ? P.ids + plane * fr[k] : nullptr, genC, genZ, e1[k].x, lane);
 				}
 			continue;
 		}
@@ -817,7 +863,7 @@ __global__ void __launch_bounds__(128, FUSED ? DTR_FUSED_CTAS : VIS_CTAS_PER_SM)
 		J.genZ        = genZ;
 		J.genC        = genC;
 		J.listOff     = d0.z;
-		process_region_vis<FUSED>(P, W, lane, J, shaded, next);
+		process_region_vis<FUSED, IDS>(P, W, I, lane, J, shaded, next);
 	}
 #if DTR_VIS_LANE_COUNT
 	shaded = __reduce_add_sync(0xffffffffu, shaded);
@@ -829,6 +875,8 @@ constexpr auto raster_vis_kernel = raster_opaque_kernel<false>; // visibility on
 // Visibility and resolve in ONE kernel: a region's pending pixels are shaded from shared memory as soon as
 // its walk is over, by the warp that owns it; no tag planes, no second pass over the busy tiles.
 constexpr auto raster_visres_kernel = raster_opaque_kernel<true>;
+constexpr auto raster_vis_ids_kernel    = raster_opaque_kernel<false, true>;
+constexpr auto raster_visres_ids_kernel = raster_opaque_kernel<true, true>;
 
 // Resolve: every pixel of the tiles that have primitives; a pixel that still carries a tag is shaded
 // from its triangle's record.  One CTA per busy tile (grid-stride), thread t takes pixels t + 256 k of

@@ -22,6 +22,7 @@ struct SetupParams
 	const FrameState *frames;
 	const TexDesc  *textures; // texture table: pointer and size are copied into textured records
 	Geometry        g;
+	uint32_t       *primId;   // null, or per primitive: 1 + its triangle's position in its frame (0: not a triangle) -- the id planes' value
 };
 
 constexpr int SCAN_THREADS = 64;    // small CTAs (64 x 32 registers) fit next to five resident raster CTAs
@@ -97,6 +98,11 @@ struct RasterParams
 	uint32_t            numTiles;       // filled by launch_raster
 	uint32_t            smallTilesMin;  // filled by launch_raster: busy tiles rasterised as fine-grained items
 	Geometry            g;
+	// Triangle id planes (appended: the fields above keep their offsets).  ids == null: off, and the kernels
+	// without id logic run; otherwise the IDS variants keep ids[F][H][W] next to the depth plane (every depth
+	// write also stores primId[] of the triangle that wrote it; a depth reset stores 0)
+	uint32_t           *ids;
+	const uint32_t     *primId;
 };
 
 // Per-device launch limits, queried once per context (dtr_b200_create) on ITS device: a process may
@@ -107,6 +113,8 @@ struct LaunchLimits
 	int residentCtas = 148; // raster CTAs resident on the whole device (sms x CTAs per SM)
 	int residentCtasVis = 148; // ... of the deferred pass's visibility kernel
 	int residentCtasVisRes = 148; // ... of the one-kernel form of the deferred pass (raster_visres_kernel)
+	// ... of the id-plane variants of the three (more shared memory per CTA: fewer of them per SM)
+	int residentCtasIds = 148, residentCtasVisIds = 148, residentCtasVisResIds = 148;
 };
 LaunchLimits query_launch_limits(int device);
 void         launch_init_tables(cudaStream_t s); // per-device lookup tables of the raster kernel (once per context)

@@ -2,7 +2,8 @@
 //
 // Data layout in HBM (see DESIGN.md §3):
 //   frames        colour u32[F][H][W] (0x00RRGGBB) and depth f32[F][H][W], row 0 = bottom --
-//                 exactly DTRRenderBuffer's planes (DTRendererRender.h:14-25), one pair per frame.
+//                 exactly DTRRenderBuffer's planes (DTRendererRender.h:14-25), one pair per frame;
+//                 optionally triangle ids u32[F][H][W] (dtr_b200_set_id_output), same layout.
 //   DrawItem[]    one per recorded draw call (tiny), uploaded per flush.
 //   PrimRecord[]  one 160-byte record per primitive in submission order, written by the setup
 //                 kernel, read by the raster kernel as ten 128-bit broadcast loads.
@@ -119,7 +120,8 @@ struct alignas(16) DrawItem
 	uint32_t count;
 	int32_t  texId; // < 0: untextured
 	uint32_t lightMode;
-	uint32_t pad0, pad1;
+	uint32_t triBase; // ITEM_TRIS / ITEM_MESH: position of the item's first triangle in its frame (triangle id planes)
+	uint32_t pad1;
 	// ITEM_TRIS: device pointers to p f32[count*9], color f32[count*4], uv f32[count*6] (or 0)
 	// ITEM_MESH: vertexes, texUV, normals, faces
 	// ITEM_RAW : record

@@ -251,6 +251,23 @@ int dtr_b200_band_barrier(dtr_b200_ctx *ctx);
 /* Device pointers of a frame's planes (u32[W*H], f32[W*H]) for zero-copy consumers
  * (NCCL / peer access / torch views). */
 int dtr_b200_frame_device_ptrs(dtr_b200_ctx *ctx, int frame, void **color, void **z);
+/* Triangle id planes: a third plane per frame, u32[F][H][W], row 0 at the bottom like the depth plane.
+ * A pixel holds 0 when no triangle fragment has written its depth since the frame's depth was last reset
+ * or uploaded (dtr_b200_begin_frame), else 1 + n, n the 0-based position in the frame of the triangle
+ * whose fragment last wrote depth there.  Triangles are counted in submission order since the frame's
+ * begin_frame, across flushes, every submitted one included: triangle / textured_triangle 1, triangles n,
+ * mesh and each view of mesh_views numFaces (face order).  The id changes exactly when depth does
+ * (translucent fragments write depth too); rectangles, bitmaps, lines, text and clears never touch it.
+ * With a band (set_band) only the band's rows are written; with foreign output planes
+ * (set_output_planes / open_peer_frames) the ids still go to this context's own planes.
+ *   dtr_b200_set_id_output  enable: allocate and zero the planes (DTR_B200_ERR_NOMEM if that fails);
+ *                           0: free them.  Applies to every later flush and replay.
+ *   dtr_b200_read_ids       flushes, copies frames [firstFrame, firstFrame + n) and waits
+ *   dtr_b200_frame_id_ptr   device pointer of a frame's id plane
+ * Both readers return DTR_B200_ERR_ARG when ids are off or the frame range is bad. */
+int dtr_b200_set_id_output(dtr_b200_ctx *ctx, int enable);
+int dtr_b200_read_ids(dtr_b200_ctx *ctx, int firstFrame, int n, uint32_t *hostIds);
+int dtr_b200_frame_id_ptr(dtr_b200_ctx *ctx, int frame, void **ids);
 int dtr_b200_get_stats(dtr_b200_ctx *ctx, dtr_b200_stats *out); /* syncs */
 /* How the raster stage of a pass made ONLY of opaque triangles onto frames cleared on chip runs (nothing
  * can ever be blended there: a pixel's colour is the shading of the last fragment that passed the depth
