@@ -30,10 +30,6 @@ namespace
 
 std::string g_createError;
 
-#ifndef DTR_PIPE_SETS
-#define DTR_PIPE_SETS 3
-#endif
-
 struct DevBuf
 {
 	void  *p   = nullptr;
@@ -138,7 +134,7 @@ struct dtr_b200_ctx
 		bool                rasterPending = false; // rasterDone has been recorded: the set may still be read
 		size_t              cleanBytes = 0;        // the first cleanBytes of tileCount were zeroed by the last raster kernel
 	};
-	static constexpr int PIPE_SETS = DTR_PIPE_SETS;
+	static constexpr int PIPE_SETS = 3;
 	PipeSet             sets[PIPE_SETS];
 	int                 nextReplaySet = 1;
 	bool                replayOverlap = true; // dtr_b200_set_replay_overlap

@@ -44,24 +44,7 @@ struct VisSmem
 };
 constexpr int      VIS_CTAS_PER_SM = 6;
 constexpr int      VIS_IDS_CTAS_PER_SM = 4; // the id-plane variants: what their shared memory (VisSmem + IdSmem per warp) allows
-#ifndef DTR_VIS_LANE_COUNT
-#define DTR_VIS_LANE_COUNT 1 // SetPixel calls counted per lane (no vote in the coverage step), summed once per warp
-#endif
-#ifndef DTR_VIS_SMALL_WINDOWS
-#define DTR_VIS_SMALL_WINDOWS 0 // N > 0: exact triangles whose clipped bbox is at most N 8x4 windows skip the sub-block table (measured: 8 -> +2 %, 16 -> +6 % raster time; the table path culls hidden sub-blocks, this one cannot)
-#endif
-#ifndef DTR_RESOLVE_STREAMS_EMPTY
-#define DTR_RESOLVE_STREAMS_EMPTY 0
-#endif
-#ifndef DTR_FUSED_CTAS
-#define DTR_FUSED_CTAS 6 // resident CTAs per SM the one-kernel form is compiled for
-#endif
-#ifndef DTR_FUSED_WIDE
-#define DTR_FUSED_WIDE 2 // one-kernel form: this many sub-blocks per resolve step, shaded as interleaved instruction streams (1, 2 or 4)
-#endif
-#ifndef DTR_VIS_EMPTY_SHIFT
-#define DTR_VIS_EMPTY_SHIFT 0 // (2: no gain) log2 of the untouched tiles per work item of a large launch
-#endif
+constexpr uint32_t VIS_EMPTY_SHIFT = 0; // (2: no gain) log2 of the untouched tiles per work item of a large launch
 constexpr uint32_t VIS_PENDING     = 0x80000000u;
 constexpr uint32_t VIS_OUTSIDE     = 0x40000000u; // resolve_kernel: a pixel of the tile that lies outside the frame (no colour has this bit)
 
@@ -326,10 +309,8 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 	}
 	__syncwarp();
 
-#if DTR_SUB_ZCULL && DTR_REGION_ZCULL
 	int zsub = depth_key(-FLT_MAX);
-#endif
-	uint32_t       passes  = 0; // this LANE's fragments that passed the depth test = SetPixel calls (summed at the end of the kernel)
+	uint32_t       passes  = 0; // this LANE's fragments that passed the depth test = SetPixel calls (summed once per warp at the end of the kernel: no vote in the coverage step)
 	const uint32_t laneBit = 1u << lane;
 	const uint32_t zAddrLane = (uint32_t)__cvta_generic_to_shared(W.z + lane);
 	const uint32_t cAddrLane = (uint32_t)__cvta_generic_to_shared(W.c + lane);
@@ -351,9 +332,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			const int B1 = sxo * dx1 + syo * dy1, B2 = sxo * dx2 + syo * dy2, B3 = sxo * dx3 + syo * dy3;
 			bool keep = (sxo < x1) && (sxo + SUB_W > x0) && (syo < y1) && (syo + SUB_H > y0);
 			keep = keep && ((((int)g3.x + B1) | ((int)g3.y + B2) | ((int)g3.z + B3)) >= 0);
-#if DTR_SUB_ZCULL && DTR_REGION_ZCULL
 			keep = keep && ((int)g3.w > zsub);
-#endif
 			const int      nx = min(max(x1 - sxo, 0), SUB_W), ny = min(max(y1 - syo, 0), SUB_H);
 			const uint32_t inMask = (((1u << nx) - 1u) * 0x01010101u) & (ny >= SUB_H ? 0xffffffffu : ((1u << (8 * ny)) - 1u));
 			__syncwarp();
@@ -385,69 +364,9 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			             : "r"((uint32_t)pass), "r"(za), "f"(z), "r"(ca), "r"(tag)
 			             : "memory");
 			if (IDS) asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %0, 0;\n\t@q st.shared.u32 [%1], %2;\n\t}" : : "r"((uint32_t)pass), "r"(iAddrLane + (s << 7)), "r"(id) : "memory");
-#if DTR_VIS_LANE_COUNT
 			passes += pass ? 1u : 0u;
-#else
-			passes += __popc(__ballot_sync(FULL, pass));
-#endif
 		}
 	};
-
-#if DTR_VIS_SMALL_WINDOWS
-	// exact triangle with a small bounding box: 8x4 WINDOWS laid from the bbox corner instead of the
-	// region's sub-block grid.  A 30-pixel mesh triangle (bbox ~8x8) is two windows but straddles five or
-	// six sub-blocks; and nothing is tabulated first (no classification, no table, no warp barriers).
-	// Lane (lx, ly) of a window is pixel (x0 + 8 wx + lx, y0 + 4 wy + ly): any 8x4 window of the linear
-	// sub-block layout falls on 32 different banks.  The edge functions are carried as fp32 and stepped
-	// by +8 dx / +4 dy: every value is an integer below 2^24 (the PF_EXACT bound covers the bbox grown by
-	// one window), so the sums are exact and the bits equal those of the table path.
-	auto raster_tri_small = [&](const uint4 g0, const uint4 g1, const uint4 g2, const uint4 g4, const int nwx, const int nwy, const uint32_t id) {
-		const int      x0 = g0.w & 0xFF, y0 = (g0.w >> 8) & 0xFF, x1 = (g0.w >> 16) & 0xFF, y1 = g0.w >> 24;
-		const float4   zp  = u2f4(g4); // 1/area, z1, z2-z1, z3-z1
-		const uint32_t tag = VIS_PENDING | g2.w;
-		const int      dx1 = (int)g1.x, dx2 = (int)g1.y, dx3 = (int)g1.z;
-		const int      dy1 = (int)g2.x, dy2 = (int)g2.y, dy3 = (int)g2.z;
-		const int      pxl = x0 + lx, pyl = y0 + ly; // this lane's pixel of the first window
-		float          r1 = (float)((int)g0.x + pxl * dx1 + pyl * dy1);
-		float          r2 = (float)((int)g0.y + pxl * dx2 + pyl * dy2);
-		float          r3 = (float)((int)g0.z + pxl * dx3 + pyl * dy3);
-		const float    sx1 = (float)(SUB_W * dx1), sx2 = (float)(SUB_W * dx2), sx3 = (float)(SUB_W * dx3);
-		const float    sy1 = (float)(SUB_H * dy1), sy2 = (float)(SUB_H * dy2), sy3 = (float)(SUB_H * dy3);
-		uint32_t       rowAddr = zAddrLane - 4u * (uint32_t)lane +
-		                   4u * (uint32_t)(((((pyl >> 2) * SUBS_X) + (pxl >> 3)) << 5) | ((pyl & 3) << 3) | (pxl & 7));
-		int            py = pyl;
-		__syncwarp(); // the triangle before touched these pixels through other lanes
-		for (int wy = 0; wy < nwy; wy++)
-		{
-			float      e1 = r1, e2 = r2, e3 = r3;
-			uint32_t   za = rowAddr;
-			int        px = pxl;
-			const bool rowIn = py < y1;
-			for (int wx = 0; wx < nwx; wx++)
-			{
-				const bool in = rowIn && (px < x1);
-				float      zOld = 0.0f;
-				asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %1, 0;\n\t@q ld.shared.f32 %0, [%2];\n\t}" : "+f"(zOld) : "r"((uint32_t)in), "r"(za) : "memory");
-				const bool  covered = in && ((__float_as_int(e1) | __float_as_int(e2) | __float_as_int(e3)) >= 0);
-				const float bB = e2 * zp.x, bC = e3 * zp.x;
-				const float z  = (zp.y + (bB * zp.z)) + (bC * zp.w);
-				const bool  pass = covered & (z > zOld);
-				asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %0, 0;\n\t@q st.shared.f32 [%1], %2;\n\t@q st.shared.u32 [%3], %4;\n\t}"
-				             :
-				             : "r"((uint32_t)pass), "r"(za), "f"(z), "r"(za - (uint32_t)(sizeof(uint32_t) * REGION_WORDS)), "r"(tag)
-				             : "memory");
-				if (IDS) asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %0, 0;\n\t@q st.shared.u32 [%1], %2;\n\t}" : : "r"((uint32_t)pass), "r"(iAddrLane + (za - zAddrLane)), "r"(id) : "memory");
-				passes += pass ? 1u : 0u;
-				e1 += sx1; e2 += sx2; e3 += sx3;
-				za += 32u * 4u; // the same pixel of the sub-block to the right
-				px += SUB_W;
-			}
-			r1 += sy1; r2 += sy2; r3 += sy3;
-			rowAddr += SUBS_X * 32u * 4u; // ... of the sub-block below
-			py += SUB_H;
-		}
-	};
-#endif
 
 	// inexact triangle: the row-shared replay of raster_tri_replay; fragments are shaded at once
 	auto raster_tri_replay = [&](const uint32_t pidx, const uint4 g0, const uint4 g1, const uint4 g2, const uint4 g4, const uint32_t id) {
@@ -486,20 +405,13 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 				W.z[si] = z;
 				W.c[si] = shade_opaque_now(P.prims + pidx, e1, e2, e3);
 				if (IDS) I->t[si] = id;
-#if DTR_VIS_LANE_COUNT
 				passes++;
-#endif
 			}
-#if !DTR_VIS_LANE_COUNT
-			passes += __popc(__ballot_sync(FULL, pass));
-#endif
 		}
 		__syncwarp();
 	};
 
-#if DTR_REGION_ZCULL
 	uint32_t zcState = J.genZ ? 1u : 0u;
-#endif
 	for (uint32_t base = 0; base < J.count; base += 32)
 	{
 		const uint32_t e    = base + lane;
@@ -510,20 +422,16 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			const uint32_t le = J.listOff + e;
 			pidx          = __ldg(P.lists + le);
 			const uint2 b = __ldg(P.listBounds + le);
-#if DTR_REGION_ZCULL
 			W.zk[lane]    = __ldg(P.listZ + le);
-#endif
 			const int minx = b.x & 0xFFFF, miny = b.x >> 16, maxx = b.y & 0xFFFF, maxy = b.y >> 16;
 			ov = (minx < rx1) && (maxx > gx) && (miny < ry1) && (maxy > gy);
 		}
 		uint32_t m = __ballot_sync(FULL, ov);
 		while (m)
 		{
-#if DTR_REGION_ZCULL
 			if ((zcState & 0xFFu) == 0u)
 			{
 				const float4 *z4 = reinterpret_cast<const float4 *>(W.z);
-#if DTR_SUB_ZCULL
 				int mySub = DEPTH_KEY_UNKNOWN;
 				for (int k = 0; k < regionWords / 128; k++)
 				{
@@ -537,16 +445,6 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 				}
 				zsub = mySub;
 				const int zminKey = __reduce_min_sync(FULL, mySub);
-#else
-				float4 q  = z4[lane];
-				float  zm = fminf(fminf(q.x, q.y), fminf(q.z, q.w));
-				for (int k = 1; k < regionWords / 128; k++)
-				{
-					q  = z4[lane + 32 * k];
-					zm = fminf(zm, fminf(fminf(q.x, q.y), fminf(q.z, q.w)));
-				}
-				const int zminKey = __reduce_min_sync(FULL, depth_key(zm));
-#endif
 				const uint32_t hidden  = __ballot_sync(FULL, W.zk[lane] <= zminKey) & m;
 				const uint32_t prev    = zcState >> 8;
 				const uint32_t backoff = ((uint32_t)__popc(hidden) >= ZCULL_RESET) ? 0u : (hidden ? prev : min(2u * prev + 1u, ZCULL_MAX_BACKOFF));
@@ -555,14 +453,11 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 				if (!m) break;
 			}
 			else zcState--;
-#endif
 			const bool     ing = ((m >> lane) & 1u) && (__popc(m & ltMask) < GROUP);
 			const uint32_t gm  = __ballot_sync(FULL, ing);
 			m &= ~gm;
-#if DTR_PREFETCH_NEXT_GROUP
 			if (((m >> lane) & 1u) && (__popc(m & ltMask) < GROUP))
 				asm volatile("prefetch.global.L1 [%0];" ::"l"(reinterpret_cast<const char *>(P.prims + pidx))); // (only the first 128 bytes are used here)
-#endif
 			// five quads per triangle instead of eleven: geometry and the depth plane, no shading data
 			bool  live = ing;
 			uint4 q0 = make_uint4(0, 0, 0, 0), q1 = q0, q2 = q0, q3 = q0, q4 = q0, g0 = q0;
@@ -582,13 +477,11 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 					g0.x = (uint32_t)((int)q1.x + relx * (int)q1.w + rely * (int)q2.z);
 					g0.y = (uint32_t)((int)q1.y + relx * (int)q2.x + rely * (int)q2.w);
 					g0.z = (uint32_t)((int)q1.z + relx * (int)q2.y + rely * (int)q3.x);
-#if DTR_REGION_REJECT
 					const int xa = x0, xb = x1 - 1, ya = y0, yb = y1 - 1;
 					const int m1 = (int)g0.x + max(xa * (int)q1.w, xb * (int)q1.w) + max(ya * (int)q2.z, yb * (int)q2.z);
 					const int m2 = (int)g0.y + max(xa * (int)q2.x, xb * (int)q2.x) + max(ya * (int)q2.w, yb * (int)q2.w);
 					const int m3 = (int)g0.z + max(xa * (int)q2.y, xb * (int)q2.y) + max(ya * (int)q3.x, yb * (int)q3.x);
 					live = (m1 | m2 | m3) >= 0;
-#endif
 				}
 			}
 			const uint32_t lm = __ballot_sync(FULL, live);
@@ -605,11 +498,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 				    g0.x + (uint32_t)((SUB_W - 1) * max((int)q1.w, 0) + (SUB_H - 1) * max((int)q2.z, 0)),
 				    g0.y + (uint32_t)((SUB_W - 1) * max((int)q2.x, 0) + (SUB_H - 1) * max((int)q2.w, 0)),
 				    g0.z + (uint32_t)((SUB_W - 1) * max((int)q2.y, 0) + (SUB_H - 1) * max((int)q3.x, 0)),
-#if DTR_SUB_ZCULL && DTR_REGION_ZCULL
 				    exact ? (uint32_t)W.zk[lane] : pidx);
-#else
-				    exact ? 0u : pidx);
-#endif
 				W.geo[r * 5 + 4] = q4;
 				if (IDS) I->geo[r] = __ldg(P.primId + pidx);
 			}
@@ -618,16 +507,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 			{
 				const uint4    g0r = W.geo[r * 5], g1 = W.geo[r * 5 + 1], g2 = W.geo[r * 5 + 2], g3 = W.geo[r * 5 + 3], g4 = W.geo[r * 5 + 4];
 				const uint32_t id = IDS ? I->geo[r] : 0u;
-				if (g1.w & PF_EXACT)
-				{
-#if DTR_VIS_SMALL_WINDOWS
-					const int bw = (int)((g0r.w >> 16) & 0xFF) - (int)(g0r.w & 0xFF), bh = (int)(g0r.w >> 24) - (int)((g0r.w >> 8) & 0xFF);
-					const int nwx = (bw + SUB_W - 1) / SUB_W, nwy = (bh + SUB_H - 1) / SUB_H;
-					if (nwx * nwy <= DTR_VIS_SMALL_WINDOWS) raster_tri_small(g0r, g1, g2, g4, nwx, nwy, id);
-					else
-#endif
-						raster_tri(g0r, g1, g2, g3, g4, id);
-				}
+				if (g1.w & PF_EXACT) raster_tri(g0r, g1, g2, g3, g4, id);
 				else raster_tri_replay(g3.w, g0r, g1, g2, g4, id);
 			}
 			__syncwarp();
@@ -642,10 +522,10 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 		// record, then the reference's shading); lane = pixel of a sub-block.  The lanes of an 8x4 block
 		// mostly carry one or two tags, so the record loads of a step are a few broadcast lines.
 		const int nSub = subsY * SUBS_X;
-		// DTR_FUSED_WIDE horizontally adjacent sub-blocks per step (a region has SUBS_X = 4 per row), one pixel
-		// of each per lane.  A lane with pending pixels in only some of them shades one of those again in
-		// place of the others: every lane with work runs the same code.
-		constexpr int NW = DTR_FUSED_WIDE;
+		// NW horizontally adjacent sub-blocks per step (a region has SUBS_X = 4 per row), one pixel of each
+		// per lane, shaded as interleaved instruction streams.  A lane with pending pixels in only some of
+		// them shades one of those again in place of the others: every lane with work runs the same code.
+		constexpr int NW = 2;
 		static_assert(SUBS_X % NW == 0, "a step's sub-blocks lie in one row of sub-blocks");
 		for (int s = 0; s < nSub; s += NW)
 		{
@@ -748,7 +628,7 @@ __device__ __forceinline__ void process_region_vis(const RasterParams &P, VisSme
 // two-kernel form keeps exactly the machine code it was measured with).  IDS: the variant that also keeps the
 // triangle id planes (RasterParams::ids), with 16 KB more shared memory per CTA.
 template <bool FUSED, bool IDS = false>
-__global__ void __launch_bounds__(128, IDS ? VIS_IDS_CTAS_PER_SM : (FUSED ? DTR_FUSED_CTAS : VIS_CTAS_PER_SM)) raster_opaque_kernel(RasterParams P)
+__global__ void __launch_bounds__(128, IDS ? VIS_IDS_CTAS_PER_SM : VIS_CTAS_PER_SM) raster_opaque_kernel(RasterParams P)
 {
 	__shared__ __align__(16) VisSmem sW[4];
 	IdSmem *I = nullptr;
@@ -764,24 +644,18 @@ __global__ void __launch_bounds__(128, IDS ? VIS_IDS_CTAS_PER_SM : (FUSED ? DTR_
 	const uint32_t nEmpty   = numTiles - nBusy;
 	const uint32_t nSmall   = min(nBusy, max((uint32_t)(((unsigned long long)nBusy * RASTER_SMALL_PERCENT) / 100), P.smallTilesMin));
 	const uint32_t nBig     = nBusy - nSmall;
-#if DTR_TINY_ITEMS
 	const bool     fewPrims   = *P.listTotal <= 64ull * nBusy;
 	const uint32_t smallShift = !fewPrims ? 2u : ((2 * nBusy < P.smallTilesMin) ? 4u : ((nBusy < P.smallTilesMin) ? 3u : 2u));
-#else
-	const uint32_t smallShift = 2u;
-#endif
-	// Untouched tiles are handed out FOUR per item when there are plenty: claiming an item and loading its
-	// tile entry is a dependent ~1.3 us, streaming a tile's clear values takes less (five tiles of six of
-	// the 1080p sphere views are untouched), so the four entries are loaded together and the claim is
-	// paid once.  (Claiming items ahead instead -- a ring of up to four claims per warp -- cost 12 %: the
-	// last busy regions then start late.)
+	// Untouched tiles can be handed out 1 << VIS_EMPTY_SHIFT per item when there are plenty: claiming an
+	// item and loading its tile entry is a dependent ~1.3 us, streaming a tile's clear values takes less
+	// (five tiles of six of the 1080p sphere views are untouched), so the entries of an item are loaded
+	// together and the claim is paid once.  Four per item measured no gain over one, so the shift is 0.
+	// The loops below keep their general form: written for one tile they compile to a different
+	// instruction schedule than the one that was measured.  (Claiming items ahead instead -- a ring of up
+	// to four claims per warp -- cost 12 %: the last busy regions then start late.)
 	const uint32_t warpsTotal  = gridDim.x * 4u;
-	const uint32_t emptyShift  = nEmpty >= 8u * warpsTotal ? (uint32_t)DTR_VIS_EMPTY_SHIFT : 0u;
-#if DTR_RESOLVE_STREAMS_EMPTY
-	const uint32_t emptyItems  = 0u; // the resolve kernel streams the untouched tiles
-#else
+	const uint32_t emptyShift  = nEmpty >= 8u * warpsTotal ? VIS_EMPTY_SHIFT : 0u;
 	const uint32_t emptyItems  = (nEmpty + (1u << emptyShift) - 1u) >> emptyShift;
-#endif
 	const uint32_t itemsBusy   = 2 * nBig + (nSmall << smallShift);
 	const uint32_t itemsMixed  = itemsBusy + (uint32_t)(((unsigned long long)emptyItems * (100 - RASTER_TAIL_PERCENT)) / 100);
 	const uint32_t itemsTotal  = itemsBusy + emptyItems;
@@ -804,10 +678,10 @@ __global__ void __launch_bounds__(128, IDS ? VIS_IDS_CTAS_PER_SM : (FUSED ? DTR_
 			if (lane == 0) next = atomicAdd(P.workCounter, 1u);
 			const uint32_t first = (item - b0) << emptyShift;
 			const uint32_t n     = min(1u << emptyShift, nEmpty - first);
-			uint32_t       fr[1 << DTR_VIS_EMPTY_SHIFT];
-			uint4          e1[1 << DTR_VIS_EMPTY_SHIFT];
+			uint32_t       fr[1 << VIS_EMPTY_SHIFT];
+			uint4          e1[1 << VIS_EMPTY_SHIFT];
 #pragma unroll
-			for (uint32_t k = 0; k < (1u << DTR_VIS_EMPTY_SHIFT); k++)
+			for (uint32_t k = 0; k < (1u << VIS_EMPTY_SHIFT); k++)
 				if (k < n)
 				{
 					const uint32_t slot = numTiles - 1 - (first + k);
@@ -815,7 +689,7 @@ __global__ void __launch_bounds__(128, IDS ? VIS_IDS_CTAS_PER_SM : (FUSED ? DTR_
 					e1[k] = __ldg(P.order + 2 * slot + 1);
 				}
 #pragma unroll
-			for (uint32_t k = 0; k < (1u << DTR_VIS_EMPTY_SHIFT); k++)
+			for (uint32_t k = 0; k < (1u << VIS_EMPTY_SHIFT); k++)
 				if (k < n)
 				{
 					const bool genZ = (e1[k].y & FI_Z_RESET) != 0, genC = (e1[k].y & FI_COLOR_CLEAR) != 0;
@@ -865,9 +739,7 @@ __global__ void __launch_bounds__(128, IDS ? VIS_IDS_CTAS_PER_SM : (FUSED ? DTR_
 		J.listOff     = d0.z;
 		process_region_vis<FUSED, IDS>(P, W, I, lane, J, shaded, next);
 	}
-#if DTR_VIS_LANE_COUNT
 	shaded = __reduce_add_sync(0xffffffffu, shaded);
-#endif
 	if (lane == 0 && shaded) atomicAdd(P.setPixels, (unsigned long long)shaded);
 }
 
@@ -881,83 +753,16 @@ constexpr auto raster_visres_ids_kernel = raster_opaque_kernel<true, true>;
 // Resolve: every pixel of the tiles that have primitives; a pixel that still carries a tag is shaded
 // from its triangle's record.  One CTA per busy tile (grid-stride), thread t takes pixels t + 256 k of
 // the tile, row-major: a warp reads and writes whole 128-byte row segments.
-#ifndef DTR_RESOLVE_MIN_CTAS
-#define DTR_RESOLVE_MIN_CTAS 8 // 32 registers: all 64 warps of an SM resident
-#endif
-#ifndef DTR_RESOLVE_UNROLL
-#define DTR_RESOLVE_UNROLL 8 // (2: -1 %; the tags then live in local memory)
-#endif
-#ifndef DTR_RESOLVE_BLOCKS
-#define DTR_RESOLVE_BLOCKS 0
-#endif
-#ifndef DTR_RESOLVE_PREFETCH
-#define DTR_RESOLVE_PREFETCH 0
-#endif
-#define DTR_RESOLVE_PRAGMA_(x) _Pragma(#x)
-#define DTR_RESOLVE_UNROLL_PRAGMA(n) DTR_RESOLVE_PRAGMA_(unroll n)
-__global__ void __launch_bounds__(256, DTR_RESOLVE_MIN_CTAS) resolve_kernel(ResolveParams R)
+constexpr int RESOLVE_MIN_CTAS = 8; // 32 registers: all 64 warps of an SM resident
+__global__ void __launch_bounds__(256, RESOLVE_MIN_CTAS) resolve_kernel(ResolveParams R)
 {
 	constexpr int  PER_THREAD = TILE_W * TILE_H / 256;
 	const uint32_t nBusy = *R.numBusy;
 	const size_t   plane = (size_t)R.g.width * R.g.height;
 	const bool     split = R.tags != R.color; // foreign output planes: every pixel of a busy tile is stored
-#if DTR_RESOLVE_BLOCKS
-	// a warp takes an 8x4 block of pixels (four 32-byte row segments): fewer distinct triangles per warp
-	const int      px0 = ((int)threadIdx.x >> 5) * 8 + ((int)threadIdx.x & 7), py0 = ((int)threadIdx.x >> 3) & 3;
-#else
 	const int      px0 = (int)threadIdx.x & (TILE_W - 1), py0 = (int)threadIdx.x / TILE_W; // pixel of the first of the thread's rows
-#endif
-#if DTR_RESOLVE_STREAMS_EMPTY
-	// Untouched tiles (their clear colour and depth, generated here) are streamed by this kernel, a few
-	// after every busy tile of the CTA: 64 resident warps per SM hide the item latency that the
-	// visibility kernel's 24 cannot, and the HBM write stream overlaps the shading's L2 waits.
-	const uint32_t nEmpty   = R.numTiles - nBusy;
-	const uint32_t perBusy  = nBusy ? (nEmpty + nBusy - 1u) / nBusy : 0u;
-	uint32_t       nextEmpty = blockIdx.x;
-	auto stream_tile = [&](const uint32_t e) {
-		const uint32_t slot = R.numTiles - 1u - e;
-		const uint32_t fr   = __ldg(&R.order[2 * slot].w);
-		const uint4    d1   = __ldg(R.order + 2 * slot + 1);
-		const bool     genZ = (d1.y & FI_Z_RESET) != 0, genC = (d1.y & FI_COLOR_CLEAR) != 0;
-		const int      gx0 = (int)(d1.z & 0xFFFFu) * TILE_W, gy0 = (int)(d1.z >> 16) * TILE_H;
-		uint32_t      *gC = R.color + plane * fr;
-		float         *gZ = R.depth + plane * fr;
-		const float    zInit = -FLT_MAX;
-		if ((R.g.width & 3) == 0)
-		{
-			const int xq = gx0 + ((int)threadIdx.x & 15) * 4;
-#pragma unroll
-			for (int h = 0; h < 2; h++)
-			{
-				const int yq = gy0 + ((int)threadIdx.x >> 4) + 16 * h;
-				if (xq < R.g.width && yq < R.g.height)
-				{
-					const size_t gi = (size_t)yq * R.g.width + xq;
-					if (genC) frame_store(reinterpret_cast<uint4 *>(gC + gi), make_uint4(d1.x, d1.x, d1.x, d1.x));
-					if (genZ) frame_store(reinterpret_cast<float4 *>(gZ + gi), make_float4(zInit, zInit, zInit, zInit));
-				}
-			}
-		}
-		else
-		{
-			for (int i = (int)threadIdx.x; i < TILE_W * TILE_H; i += 256)
-			{
-				const int xq = gx0 + (i & (TILE_W - 1)), yq = gy0 + i / TILE_W;
-				if (xq < R.g.width && yq < R.g.height)
-				{
-					const size_t gi = (size_t)yq * R.g.width + xq;
-					if (genC) gC[gi] = d1.x;
-					if (genZ) gZ[gi] = zInit;
-				}
-			}
-		}
-	};
-#endif
 	for (uint32_t slot = blockIdx.x; slot < nBusy; slot += gridDim.x)
 	{
-#if DTR_RESOLVE_STREAMS_EMPTY
-		for (uint32_t j = 0; j < perBusy && nextEmpty < nEmpty; j++, nextEmpty += gridDim.x) stream_tile(nextEmpty);
-#endif
 		const uint4 d0 = __ldg(R.order + 2 * slot), d1 = __ldg(R.order + 2 * slot + 1);
 		const int   x = (int)(d1.z & 0xFFFFu) * TILE_W + px0, yTop = (int)(d1.z >> 16) * TILE_H + py0;
 		const size_t    pix = plane * d0.w + (size_t)yTop * R.g.width + x;
@@ -972,18 +777,8 @@ __global__ void __launch_bounds__(256, DTR_RESOLVE_MIN_CTAS) resolve_kernel(Reso
 			const int y = yTop + k * (256 / TILE_W);
 			v[k] = (x < R.g.width && y < R.g.height) ? __ldcs(tag + (size_t)k * (256 / TILE_W) * R.g.width) : VIS_OUTSIDE;
 		}
-#if DTR_RESOLVE_PREFETCH
-		// the records the thread is going to read, on their way into L1 while the first pixel is shaded
-#pragma unroll
-		for (int k = 0; k < PER_THREAD; k++)
-			if (v[k] & VIS_PENDING)
-			{
-				const char *rp = reinterpret_cast<const char *>(R.prims + (v[k] & ~VIS_PENDING));
-				asm volatile("prefetch.global.L1 [%0];" ::"l"(rp));
-				asm volatile("prefetch.global.L1 [%0];" ::"l"(rp + 128));
-			}
-#endif
-		DTR_RESOLVE_UNROLL_PRAGMA(DTR_RESOLVE_UNROLL)
+		// (unroll 2: -1 %; the tags then live in local memory)
+#pragma unroll 8
 		for (int k = 0; k < PER_THREAD; k++)
 		{
 			if (!(v[k] & VIS_PENDING))
@@ -1003,7 +798,4 @@ __global__ void __launch_bounds__(256, DTR_RESOLVE_MIN_CTAS) resolve_kernel(Reso
 			frame_store_u32(col + (size_t)k * (256 / TILE_W) * R.g.width, shade_opaque_from_record(rec, (float)E1, (float)E2, (float)E3));
 		}
 	}
-#if DTR_RESOLVE_STREAMS_EMPTY
-	for (; nextEmpty < nEmpty; nextEmpty += gridDim.x) stream_tile(nextEmpty);
-#endif
 }

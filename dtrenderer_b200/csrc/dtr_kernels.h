@@ -142,8 +142,8 @@ struct ResolveParams
 	const PrimRecord *prims;
 	const uint4      *order;   // tile descriptors in work order: the busy tiles are the first *numBusy
 	const uint32_t   *numBusy;
-	float            *depth;    // [F][H][W] (only written: the clear values of untouched tiles, DTR_RESOLVE_STREAMS_EMPTY)
-	uint32_t          numTiles; // tiles of the pass (busy + untouched)
+	uint32_t          numTiles; // tiles of the pass (busy + untouched).  Not read by resolve_kernel; it keeps g.width at
+	                            // 4 mod 8 bytes, where the kernel loads it with the instruction schedule that was measured
 	Geometry          g;
 };
 

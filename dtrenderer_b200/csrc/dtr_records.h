@@ -19,28 +19,16 @@ namespace dtr
 // single warps; a region is 32 sub-blocks of 8x4 pixels (one sub-block per lane when a triangle is
 // classified against the region, one pixel per lane when a sub-block is rasterised).
 constexpr int TILE_W      = 64;
-#ifndef DTR_TILE_H
-#define DTR_TILE_H 32
-#endif
-constexpr int TILE_H      = DTR_TILE_H; // 32 (the only height the round-2 raster kernel supports, see its static_assert)
+constexpr int TILE_H      = 32; // the only height the round-2 raster kernel supports, see its static_assert
 constexpr int REGION_W    = 32;
 constexpr int REGION_H    = TILE_H;
 constexpr int SUB_W       = 8;
 constexpr int SUB_H       = 4;
-// Warp pairs (see dtr_kernels.cu): a raster CTA is four producer warps + four consumer warps, four CTAs per SM
+// A raster CTA is four warps, each with its own region (see WarpSmem in dtr_kernels.cu); five CTAs per SM
 constexpr int RASTER_THREADS = 128;
-#ifndef DTR_RASTER_CTAS
-#define DTR_RASTER_CTAS 5
-#endif
-#ifndef DTR_RASTER_TAIL
-#define DTR_RASTER_TAIL 10
-#endif
-constexpr int RASTER_TAIL_PERCENT = DTR_RASTER_TAIL; // share of the untouched tiles kept for the end of the launch
-#ifndef DTR_RASTER_SMALL
-#define DTR_RASTER_SMALL 5
-#endif
-constexpr int RASTER_SMALL_PERCENT = DTR_RASTER_SMALL; // share of the busy tiles rasterised as four 32x16 items
-constexpr int RASTER_CTAS_PER_SM = DTR_RASTER_CTAS; // 5 x 4 warps per SM, each warp with 10.4 KB of shared memory
+constexpr int RASTER_TAIL_PERCENT = 10; // share of the untouched tiles kept for the end of the launch
+constexpr int RASTER_SMALL_PERCENT = 5; // share of the busy tiles rasterised as four 32x16 items
+constexpr int RASTER_CTAS_PER_SM = 5; // 5 x 4 warps per SM, each warp with 10.4 KB of shared memory
 // Frames with many primitives are binned in segments of BIN_SEG primitives: the setup kernel counts
 // per (tile, segment), so that one CTA per (frame, tile row, segment) can write its part of every
 // tile list independently and the lists still come out in submission order.

@@ -1,4 +1,4 @@
-# A/B of kernel variants on the GPU box: build variants/libdtr_<name>.so (same sources, other -D flags or edits), then
+# A/B of kernel variants on the GPU box: build variants/libdtr_<name>.so (from edited sources), then
 # `gpurun -- bash tools/ab_variants.sh <name>...`; the library under test is selected with DTR_B200_LIB.
 # Every line is parity checked by bench.py itself (a wrong frame exits non-zero and prints PARITY FAILURE).
 cd /root/repo
