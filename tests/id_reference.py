@@ -31,6 +31,13 @@ class IdOracle:
         self._ids[:] = 0
         self._n = 0
 
+    def upload(self, color, z):
+        """Start from caller-supplied planes, as begin_frame(color=, z=) does: the ids and the count restart."""
+        self.o.color()[:] = color
+        self._z[:] = np.asarray(z, np.float32).view(np.uint32)  # bit copy: NaN payloads stay as they are
+        self._seen[:] = self._z
+        self.reset_ids()
+
     def _after_triangle(self):
         self._n += 1
         changed = self._z != self._seen
