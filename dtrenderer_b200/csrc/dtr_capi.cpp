@@ -606,10 +606,12 @@ int do_flush(dtr_b200_ctx *c)
 	// into another GPU's frame -- the one-kernel form stores finished regions straight to the output; in
 	// the two-kernel form the visibility kernel leaves its tags in this context's own colour planes and
 	// the resolve kernel stores every pixel of the busy tiles to the output.  Nothing is ever read back
-	// over NVLink.)
+	// over NVLink.)  A clear colour with bit 31 set would read as a pending tag at the pixels no triangle
+	// covers (VIS_PENDING): such a pass takes the single kernel, which gives the same frames.
 	{
 		bool deferred = c->opaqueStage != DTR_B200_OPAQUE_SINGLE_KERNEL && numItems > 0;
-		for (uint32_t s2 = 0; s2 < numActive && deferred; s2++) deferred = (fs[s2].init & FI_COLOR_CLEAR) != 0;
+		for (uint32_t s2 = 0; s2 < numActive && deferred; s2++)
+			deferred = (fs[s2].init & FI_COLOR_CLEAR) != 0 && (fs[s2].clearPacked & VIS_PENDING) == 0;
 		for (uint32_t i = 0; i < numItems && deferred; i++) deferred = c->rec[i].item.type != ITEM_RAW && c->rec[i].opaque;
 		c->last.deferred  = deferred;
 		c->last.oneKernel = deferred && c->opaqueStage == DTR_B200_OPAQUE_ONE_KERNEL;

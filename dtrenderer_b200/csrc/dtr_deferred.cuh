@@ -45,7 +45,6 @@ struct VisSmem
 constexpr int      VIS_CTAS_PER_SM = 6;
 constexpr int      VIS_IDS_CTAS_PER_SM = 4; // the id-plane variants: what their shared memory (VisSmem + IdSmem per warp) allows
 constexpr uint32_t VIS_EMPTY_SHIFT = 0; // (2: no gain) log2 of the untouched tiles per work item of a large launch
-constexpr uint32_t VIS_PENDING     = 0x80000000u;
 constexpr uint32_t VIS_OUTSIDE     = 0x40000000u; // resolve_kernel: a pixel of the tile that lies outside the frame (no colour has this bit)
 
 // The reference's per-fragment arithmetic after the depth test for an OPAQUE fragment (SlowTriangle

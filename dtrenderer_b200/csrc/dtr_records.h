@@ -136,6 +136,13 @@ enum FrameInit : uint32_t
 	FI_COLOR_CLEAR = 1u << 1, // colour starts at clearPacked, generated on chip (no read)
 };
 
+// The deferred opaque stage (dtr_deferred.cuh) tells a pixel whose shading is still pending from a finished
+// one by bit 31 of its colour word: 0x80000000 | primitive index.  Shaded colours never have it (their top
+// byte is 0).  A clear colour can: DTRRender_Clear packs (int32)(c * 255) with shifts, so a channel at or
+// below -1/255 reaches bit 31, and so do some large ones (red 130; blue 1e10, +-inf or NaN).
+// The host runs a pass whose frames clear to such a colour through the single raster kernel.
+constexpr uint32_t VIS_PENDING = 0x80000000u;
+
 struct FrameState
 {
 	uint32_t init;

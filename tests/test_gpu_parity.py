@@ -330,7 +330,9 @@ def test_null_arguments_are_silent_noops(built):
 
 
 def test_device_arithmetic_selftest(built):
-    """The blend's branch-free sqrt equals IEEE sqrtf on every float in [2^-60, 4)."""
+    """The blend's branch-free sqrt equals IEEE sqrtf on every float in [2^-60, 4), and the output byte
+    (out_byte) equals the reference's `(v == 0 ? 0 : sqrtf(v)) * 255`, clamped at 255 and truncated with NaN
+    stored as 0, on all 2^32 float bit patterns: +-inf, NaNs, negative and denormal inputs included."""
     r = _renderer(64, 48)
     assert r.selftest() == 0
 

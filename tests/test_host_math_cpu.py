@@ -45,17 +45,37 @@ def _fa(v):
     return a, a.ctypes.data_as(_f)
 
 
+# Clears outside [0, 1] and the words they pack to: (int32)(c * 255) spills into the neighbouring channels
+# and the top byte.  Those with bit 31 set would read as pending tags in the deferred opaque stage
+# (VIS_PENDING, dtr_records.h); tests/test_gpu_colour_range.py renders them.
+CLEAR_WORDS = {(0.3, 0.3, 0.7): 0x004C4CB2, (1.5, 1.2, 2.0): 0x017F33FE, (0.0, 0.0, 1e10): 0x80000000,
+               (-0.01, 0.0, 0.0): 0xFFFE0000, (0.0, 0.0, -0.004): 0xFFFFFFFF, (0.0, -1.0, 0.0): 0xFFFF0100,
+               (130.0, 0.0, 0.0): 0x817E0000, (np.nan, 0.0, 0.0): 0, (np.inf, 0.0, 0.0): 0,
+               (0.0, 1 / 255, 1e10): 0x80000100}
+CLEAR_CHANNELS = [-np.inf, -1e10, -130.0, -1.0, -0.004, -0.0, 0.0, 0.5, 1.0, float(np.nextafter(np.float32(1), np.float32(2))),
+                  2.0, 128.5, 128.51, 130.0, 257.0, 33000.0, 1e5, 1e10, np.inf, np.nan]
+
+
 def test_clear_colour_packing_matches_reference(shim):
-    """DTRRender_Clear's truncating pack (DTRendererRender.cpp:1801-1811)."""
+    """DTRRender_Clear's truncating pack (DTRendererRender.cpp:1801-1811), in [0, 1] and over the whole float
+    range: negative channels, channels > 1 and >= 128.5, 1e10, +-inf and NaN, every combination of those in
+    the three channels, and the words of CLEAR_WORDS."""
     rng = np.random.default_rng(5)
     o = _oracle(4, 3)
     cases = [rng.random(3) for _ in range(1500)]
     cases += [(1.0, 1.0, 1.0), (0.0, 0.0, 0.0), (0.999999, 0.5, 0.003921569), (np.nextafter(np.float32(1), np.float32(0)),) * 3,
               (1 / 255, 2 / 255, 254 / 255), (0.5019608, 0.25, 0.75)]
+    cases += list(CLEAR_WORDS)
+    cases += [(r, g, b) for r in CLEAR_CHANNELS for g in CLEAR_CHANNELS for b in CLEAR_CHANNELS]
+    cases += list(rng.uniform(-300, 300, (500, 3)))
+    cases += list(rng.choice([-1, 1], (500, 3)) * 10.0 ** rng.uniform(-4, 12, (500, 3)))
     for rgb in cases:
         a, p = _fa(rgb)
         o.clear(tuple(float(x) for x in a))
         assert int(o.color()[0, 0]) == shim.hm_pack_clear(p), rgb
+    for rgb, word in CLEAR_WORDS.items():
+        a, p = _fa(rgb)
+        assert shim.hm_pack_clear(p) == word, (rgb, hex(word))
 
 
 def _rect(shim, w, h, mn, mx, rot, anchor, scale, color):
