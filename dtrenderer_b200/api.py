@@ -89,6 +89,8 @@ SYMBOLS = [
     ("dtr_b200_read_frames_async", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     ("dtr_b200_wait_reads", C.c_int, [C.c_void_p]),
     ("dtr_b200_read_frames_bgr24_async", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    ("dtr_b200_set_readback_resolve", C.c_int, [C.c_void_p, C.c_int]),
+    ("dtr_b200_resolve_frames", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     ("dtr_b200_export_frames", C.c_int, [C.c_void_p, _u8, _u8]),
     ("dtr_b200_open_peer_frames", C.c_int, [C.c_void_p, _u8, _u8]),
     ("dtr_b200_set_output_planes", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -168,12 +170,13 @@ class Renderer:
 
     def __init__(self, width, height, num_frames=1, device=0):
         self.lib = load_library()
-        self.width, self.height, self.num_frames = width, height, num_frames
+        self.width, self.height, self.num_frames, self.device = width, height, num_frames, device
         h = C.c_void_p()
         rc = self.lib.dtr_b200_create(device, width, height, num_frames, C.byref(h))
         if rc != 0:
             raise DtrError(f"dtr_b200_create failed ({rc}): {self.lib.dtr_b200_last_error(None).decode()}")
         self.ctx = h
+        self.resolve = 1  # readback resolve factor (set_readback_resolve)
         self._tex = {}    # id(array) -> (texId, array)
         self._mesh = {}   # (id(mesh dict), texId) -> meshId
         self._font = {}   # id(atlas) -> (fontId, font)
@@ -317,10 +320,36 @@ class Renderer:
     def sync(self):
         self._ck(self.lib.dtr_b200_sync(self.ctx))
 
+    @property
+    def out_shape(self):
+        """(rows, columns) of a frame as the readbacks return it: the sample size over the resolve factor."""
+        return self.height // self.resolve, self.width // self.resolve
+
+    def set_readback_resolve(self, k):
+        """Every readback returns frames of (W/k) x (H/k), each pixel resolved on the device from a k x k block of
+        samples (see dtr_b200_set_readback_resolve); draw calls, uploads and device pointers stay at W x H."""
+        self._ck(self.lib.dtr_b200_set_readback_resolve(self.ctx, int(k)))
+        self.resolve = int(k)
+
+    def resolve_frames_tensors(self, first=0, n=1, ids=False):
+        """Resolved colour (int32, the view multigpu.frame_tensors uses), depth (float32) and, with ids=True, ids
+        (int32) of frames [first, first + n) as new torch tensors [n, H/k, W/k] on this context's device, filled in
+        stream order on the context's stream (dtr_b200_resolve_frames)."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        shape = (n, *self.out_shape)
+        col = torch.empty(shape, dtype=torch.int32, device=dev)
+        dep = torch.empty(shape, dtype=torch.float32, device=dev)
+        idp = torch.empty(shape, dtype=torch.int32, device=dev) if ids else None
+        self._ck(self.lib.dtr_b200_resolve_frames(self.ctx, first, n, C.c_void_p(col.data_ptr()), C.c_void_p(dep.data_ptr()),
+                                                  C.c_void_p(idp.data_ptr()) if ids else None))
+        self.sync()
+        return (col, dep, idp) if ids else (col, dep)
+
     def end_frame(self, frame=0, want_z=True, color_out=None, z_out=None):
-        """Flush and read the frame back: returns (colour u32[H,W], depth f32[H,W] or None)."""
-        col = color_out if color_out is not None else np.empty((self.height, self.width), np.uint32)
-        z = z_out if z_out is not None else (np.empty((self.height, self.width), np.float32) if want_z else None)
+        """Flush and read the frame back: returns (colour u32[H/k,W/k], depth f32[H/k,W/k] or None)."""
+        col = color_out if color_out is not None else np.empty(self.out_shape, np.uint32)
+        z = z_out if z_out is not None else (np.empty(self.out_shape, np.float32) if want_z else None)
         self._ck(self.lib.dtr_b200_end_frame(self.ctx, frame, col.ctypes.data_as(C.c_void_p),
                                              z.ctypes.data_as(C.c_void_p) if z is not None else None))
         return col, z
@@ -343,11 +372,11 @@ class Renderer:
 
     def bgr24_pitch(self):
         """Row pitch in bytes of the 24-bit DIB rows written by read_frames_bgr24_async_ptr."""
-        return (3 * self.width + 3) & ~3
+        return (3 * (self.width // self.resolve) + 3) & ~3
 
     def read_frames_bgr24_async_ptr(self, first, n, bgr_ptr):
         """Flush, pack n colour planes into 24-bit bottom-up DIBs on the device and enqueue their
-        readback (n * bgr24_pitch() * height bytes of page-locked memory); wait_reads() completes it."""
+        readback (n * bgr24_pitch() * out_shape[0] bytes of page-locked memory); wait_reads() completes it."""
         self._ck(self.lib.dtr_b200_read_frames_bgr24_async(self.ctx, first, n, C.c_void_p(bgr_ptr)))
 
     def wait_reads(self):
@@ -408,8 +437,8 @@ class Renderer:
         self._ck(self.lib.dtr_b200_set_id_output(self.ctx, 1 if on else 0))
 
     def read_ids(self, first=0, n=1):
-        """Flush and read the id planes of frames [first, first + n): u32[n, H, W]."""
-        out = np.empty((n, self.height, self.width), np.uint32)
+        """Flush and read the id planes of frames [first, first + n): u32[n, H/k, W/k]."""
+        out = np.empty((n, *self.out_shape), np.uint32)
         self._ck(self.lib.dtr_b200_read_ids(self.ctx, first, n, out.ctypes.data_as(C.c_void_p)))
         return out
 

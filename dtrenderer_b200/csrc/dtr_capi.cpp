@@ -72,12 +72,13 @@ struct dtr_b200_ctx
 	// by renderDone; copyDone lets a later flush that renders into frames still being read wait
 	cudaStream_t copyStream = nullptr;
 	cudaEvent_t  renderDone = nullptr, copyDone = nullptr;
-	// 24-bit presentation readback (dtr_b200_read_frames_bgr24_async): two device staging buffers
-	// used in turn, so that packing the next batch does not wait for the previous transfer
+	// 24-bit presentation readback (dtr_b200_read_frames_bgr24_async) and resolved readbacks: two device
+	// staging buffers used in turn, so that packing the next batch does not wait for the previous transfer
 	DevBuf       packStage[2];
 	cudaEvent_t  packFree[2] = {nullptr, nullptr}; // the D2H copy out of packStage[k] has finished
 	int          packTurn    = 0;
 	int          readLo = 0, readHi = 0; // frames [readLo, readHi) have reads in flight
+	int          resolve = 1; // readback resolve factor k (dtr_b200_set_readback_resolve)
 	struct FontHost
 	{
 		uint8_t                         *dAtlas = nullptr;
@@ -1066,6 +1067,98 @@ int dtr_b200_sync(dtr_b200_ctx *c)
 	return DTR_B200_OK;
 }
 
+namespace
+{
+// The next of the two staging buffers, grown to `bytes`; the context's stream waits until the previous
+// transfer out of it has finished.  *turn: its index, for packFree.
+int acquire_stage(dtr_b200_ctx *c, size_t bytes, int *turn)
+{
+	const int k = c->packTurn;
+	c->packTurn ^= 1;
+	if (!c->packFree[k]) CU(cudaEventCreateWithFlags(&c->packFree[k], cudaEventDisableTiming));
+	else CU(cudaStreamWaitEvent(c->stream, c->packFree[k], 0)); // the previous transfer out of this buffer
+	if (bytes > c->packStage[k].cap)
+	{
+		CU(cudaStreamSynchronize(c->copyStream)); // ensure_dev frees the old buffer
+		int rc = ensure_dev(c, c->packStage[k], bytes);
+		if (rc) return rc;
+	}
+	*turn = k;
+	return DTR_B200_OK;
+}
+
+// Resolves frames [first, first + n) at the context's factor into device memory (each output may be null),
+// in stream order.  It reads the planes the unresolved readbacks copy.
+int resolve_into(dtr_b200_ctx *c, int first, int n, uint32_t *color, float *z, uint32_t *ids)
+{
+	const size_t       plane = (size_t)c->width * c->height;
+	FrameResolveParams P{};
+	P.color    = c->outColor + plane * first;
+	P.depth    = c->outDepth + plane * first;
+	P.ids      = c->dIds ? c->dIds + plane * first : nullptr;
+	P.outColor = color;
+	P.outDepth = z;
+	P.outIds   = ids;
+	P.width    = c->width;
+	P.height   = c->height;
+	P.frames   = n;
+	launch_resolve_frames(P, c->resolve, c->stream);
+	CU(cudaGetLastError());
+	return DTR_B200_OK;
+}
+
+// The synchronous readbacks at k > 1 (after the flush): resolve into a staging buffer, copy out, wait
+int read_resolved(dtr_b200_ctx *c, int first, int n, uint32_t *hostColor, float *hostZ, uint32_t *hostIds)
+{
+	const size_t bytes = (size_t)(c->width / c->resolve) * (c->height / c->resolve) * n * sizeof(uint32_t);
+	void *const  host[3] = {hostColor, hostZ, hostIds};
+	const int    planes  = (hostColor != nullptr) + (hostZ != nullptr) + (hostIds != nullptr);
+	if (planes)
+	{
+		int turn = 0, rc = acquire_stage(c, bytes * planes, &turn);
+		if (rc) return rc;
+		uint8_t *dev[3] = {nullptr, nullptr, nullptr}, *next = static_cast<uint8_t *>(c->packStage[turn].p);
+		for (int i = 0; i < 3; i++)
+			if (host[i])
+			{
+				dev[i] = next;
+				next += bytes;
+			}
+		rc = resolve_into(c, first, n, (uint32_t *)dev[0], (float *)dev[1], (uint32_t *)dev[2]);
+		if (rc) return rc;
+		for (int i = 0; i < 3; i++)
+			if (host[i]) CU(cudaMemcpyAsync(host[i], dev[i], bytes, cudaMemcpyDeviceToHost, c->stream));
+	}
+	CU(cudaStreamSynchronize(c->stream));
+	return DTR_B200_OK;
+}
+} // namespace
+
+int dtr_b200_set_readback_resolve(dtr_b200_ctx *c, int k)
+{
+	if (!c) return DTR_B200_ERR_ARG;
+	if (k < 1 || k > 4 || c->width % k || c->height % k)
+		return fail(c, DTR_B200_ERR_ARG, "resolve factor must be in 1..4 and divide the frame's width and height");
+	c->resolve = k;
+	return DTR_B200_OK;
+}
+
+int dtr_b200_resolve_frames(dtr_b200_ctx *c, int first, int n, void *color, void *z, void *ids)
+{
+	if (!c) return DTR_B200_ERR_ARG;
+	if (ids && !c->dIds) return fail(c, DTR_B200_ERR_ARG, "triangle id output is off (dtr_b200_set_id_output)");
+	if (n <= 0 || !valid_frame(c, first) || !valid_frame(c, first + n - 1)) return fail(c, DTR_B200_ERR_ARG, "frame range out of bounds");
+	CU(cudaSetDevice(c->device));
+	int rc = do_flush(c);
+	if (rc) return rc;
+	if (c->resolve > 1) return resolve_into(c, first, n, (uint32_t *)color, (float *)z, (uint32_t *)ids);
+	const size_t bytes = (size_t)c->width * c->height * n * sizeof(uint32_t), off = (size_t)c->width * c->height * first;
+	if (color) CU(cudaMemcpyAsync(color, c->outColor + off, bytes, cudaMemcpyDeviceToDevice, c->stream));
+	if (z) CU(cudaMemcpyAsync(z, c->outDepth + off, bytes, cudaMemcpyDeviceToDevice, c->stream));
+	if (ids) CU(cudaMemcpyAsync(ids, c->dIds + off, bytes, cudaMemcpyDeviceToDevice, c->stream));
+	return DTR_B200_OK;
+}
+
 int dtr_b200_end_frame(dtr_b200_ctx *c, int frame, uint32_t *hostColor, float *hostZ)
 {
 	if (!c) return DTR_B200_ERR_ARG;
@@ -1073,6 +1166,7 @@ int dtr_b200_end_frame(dtr_b200_ctx *c, int frame, uint32_t *hostColor, float *h
 	CU(cudaSetDevice(c->device));
 	int rc = do_flush(c);
 	if (rc) return rc;
+	if (c->resolve > 1) return read_resolved(c, frame, 1, hostColor, hostZ, nullptr);
 	size_t plane = (size_t)c->width * c->height;
 	if (hostColor)
 		CU(cudaMemcpyAsync(hostColor, c->outColor + plane * frame, plane * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
@@ -1088,6 +1182,7 @@ int dtr_b200_read_frames(dtr_b200_ctx *c, int first, int n, uint32_t *hostColor,
 	CU(cudaSetDevice(c->device));
 	int rc = do_flush(c);
 	if (rc) return rc;
+	if (c->resolve > 1) return read_resolved(c, first, n, hostColor, hostZ, nullptr);
 	size_t plane = (size_t)c->width * c->height;
 	if (hostColor)
 		CU(cudaMemcpyAsync(hostColor, c->outColor + plane * first, plane * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
@@ -1104,6 +1199,23 @@ int dtr_b200_read_frames_async(dtr_b200_ctx *c, int first, int n, uint32_t *host
 	CU(cudaSetDevice(c->device));
 	int rc = do_flush(c);
 	if (rc) return rc;
+	if (c->resolve > 1)
+	{
+		// resolve into a staging buffer, copy from there: the frames are free once the resolve kernel has run
+		const size_t bytes  = (size_t)(c->width / c->resolve) * (c->height / c->resolve) * n * sizeof(uint32_t);
+		const int    planes = (hostColor != nullptr) + (hostZ != nullptr);
+		if (!planes) return DTR_B200_OK;
+		int turn = 0;
+		if ((rc = acquire_stage(c, bytes * planes, &turn))) return rc;
+		uint8_t *dev = static_cast<uint8_t *>(c->packStage[turn].p), *devZ = hostColor ? dev + bytes : dev;
+		if ((rc = resolve_into(c, first, n, hostColor ? (uint32_t *)dev : nullptr, hostZ ? (float *)devZ : nullptr, nullptr))) return rc;
+		CU(cudaEventRecord(c->renderDone, c->stream));
+		CU(cudaStreamWaitEvent(c->copyStream, c->renderDone, 0));
+		if (hostColor) CU(cudaMemcpyAsync(hostColor, dev, bytes, cudaMemcpyDeviceToHost, c->copyStream));
+		if (hostZ) CU(cudaMemcpyAsync(hostZ, devZ, bytes, cudaMemcpyDeviceToHost, c->copyStream));
+		CU(cudaEventRecord(c->packFree[turn], c->copyStream));
+		return DTR_B200_OK;
+	}
 	size_t plane = (size_t)c->width * c->height;
 	CU(cudaEventRecord(c->renderDone, c->stream));
 	CU(cudaStreamWaitEvent(c->copyStream, c->renderDone, 0));
@@ -1134,20 +1246,15 @@ int dtr_b200_read_frames_bgr24_async(dtr_b200_ctx *c, int first, int n, uint8_t 
 	CU(cudaSetDevice(c->device));
 	int rc = do_flush(c);
 	if (rc) return rc;
-	const size_t pitch = ((size_t)c->width * 3 + 3) & ~(size_t)3, rows = (size_t)n * c->height, bytes = pitch * rows;
-	const int    k     = c->packTurn;
-	c->packTurn ^= 1;
-	if (!c->packFree[k]) CU(cudaEventCreateWithFlags(&c->packFree[k], cudaEventDisableTiming));
-	else CU(cudaStreamWaitEvent(c->stream, c->packFree[k], 0)); // the previous transfer out of this buffer
-	if (bytes > c->packStage[k].cap)
-	{
-		CU(cudaStreamSynchronize(c->copyStream)); // ensure_dev frees the old buffer
-		rc = ensure_dev(c, c->packStage[k], bytes);
-		if (rc) return rc;
-	}
+	const int    ow = c->width / c->resolve;
+	const size_t pitch = ((size_t)ow * 3 + 3) & ~(size_t)3, rows = (size_t)n * (c->height / c->resolve), bytes = pitch * rows;
+	int          k = 0;
+	if ((rc = acquire_stage(c, bytes, &k))) return rc;
 	// the frames are free again as soon as the pack kernel has run (same stream as the rendering)
-	launch_pack_bgr24(c->outColor + (size_t)c->width * c->height * first, static_cast<uint32_t *>(c->packStage[k].p), c->width, rows,
-	                  (int)(pitch / 4), c->stream);
+	const uint32_t *frames = c->outColor + (size_t)c->width * c->height * first;
+	if (c->resolve > 1)
+		launch_resolve_pack_bgr24(frames, static_cast<uint32_t *>(c->packStage[k].p), c->width, c->resolve, rows, (int)(pitch / 4), c->stream);
+	else launch_pack_bgr24(frames, static_cast<uint32_t *>(c->packStage[k].p), c->width, rows, (int)(pitch / 4), c->stream);
 	CU(cudaGetLastError());
 	CU(cudaEventRecord(c->renderDone, c->stream));
 	CU(cudaStreamWaitEvent(c->copyStream, c->renderDone, 0));
@@ -1406,6 +1513,7 @@ int dtr_b200_read_ids(dtr_b200_ctx *c, int first, int n, uint32_t *hostIds)
 	CU(cudaSetDevice(c->device));
 	int rc = do_flush(c);
 	if (rc) return rc;
+	if (c->resolve > 1) return read_resolved(c, first, n, nullptr, nullptr, hostIds);
 	const size_t plane = (size_t)c->width * c->height;
 	CU(cudaMemcpyAsync(hostIds, c->dIds + plane * first, plane * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
 	CU(cudaStreamSynchronize(c->stream));

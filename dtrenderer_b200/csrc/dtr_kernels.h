@@ -163,4 +163,19 @@ void launch_raster_deferred(const RasterParams &P, const LaunchLimits &L, cudaSt
 void launch_premultiply(uint32_t *pixels, size_t count, cudaStream_t s);
 void launch_pack_bgr24(const uint32_t *color, uint32_t *out, int width, size_t rows, int pitchWords, cudaStream_t s);
 
+// Readback resolve of n frames at factor k (2..4, dividing width and height): resolve_frames_kernel<k, ...>
+struct FrameResolveParams
+{
+	const uint32_t *color; // sample planes [frames][height][width] (read where the matching output is wanted)
+	const float    *depth; // read when outDepth or outIds is wanted
+	const uint32_t *ids;   // read when outIds is wanted
+	uint32_t       *outColor; // [frames][height/k][width/k], each may be null
+	float          *outDepth;
+	uint32_t       *outIds;
+	int             width, height, frames;
+};
+void launch_resolve_frames(const FrameResolveParams &P, int k, cudaStream_t s);
+// resolve_pack_bgr24_kernel<k, ...>: the colour of outRows output rows resolved and packed as launch_pack_bgr24 packs
+void launch_resolve_pack_bgr24(const uint32_t *color, uint32_t *out, int width, int k, size_t outRows, int pitchWords, cudaStream_t s);
+
 } // namespace dtr

@@ -212,6 +212,33 @@ int dtr_b200_wait_reads(dtr_b200_ctx *ctx);
  * hostBgr: n * pitch * H bytes, page-locked; valid after dtr_b200_wait_reads.  The frames may be
  * rendered into again at once (the pack runs in stream order, the transfer reads a staging copy). */
 int dtr_b200_read_frames_bgr24_async(dtr_b200_ctx *ctx, int firstFrame, int n, uint8_t *hostBgr);
+/* Supersampled output: a context has a READBACK RESOLVE FACTOR k, default 1.  Render into a kW x kH
+ * context and every host readback -- dtr_b200_end_frame, dtr_b200_read_frames, dtr_b200_read_frames_async,
+ * dtr_b200_read_frames_bgr24_async (pitch ((3*W/k + 3) & ~3)) and dtr_b200_read_ids -- returns frames of
+ * (W/k) x (H/k), row 0 at the bottom as before.  Output pixel (X, Y) is made on the device from the block of
+ * samples [kX, kX+k) x [kY, kY+k) of the frame's planes:
+ *   colour  each of the four bytes of the 0x00RRGGBB word separately (the X byte too, which clear colours
+ *           outside [0, 1] can set): the integer square root of the integer mean, rounded down, of the squared
+ *           sample bytes, floor(sqrt(floor(sum(b^2) / k^2))) -- the largest v with v^2 k^2 <= sum(b^2).  This is
+ *           the mean in the reference's gamma-2 linear space, encoded back with truncation; a block of equal
+ *           words resolves to that word.
+ *   depth   one sample per block: scanning the block row by row from its bottom-left sample, the first sample
+ *   and id  is taken and replaced only by a sample whose depth compares > (IEEE) with the current one (ties
+ *           and NaN keep the earlier sample).  Depth is the chosen sample's bits, the id the chosen sample's
+ *           id: both always come from the same fragment.
+ * k = 1 is the plain readback (the same copies, no resolve kernel).  Uploads (dtr_b200_begin_frame), device
+ * pointers (dtr_b200_frame_device_ptrs, dtr_b200_frame_id_ptr), every draw call and dtr_b200_get_stats stay at
+ * sample resolution: setPixels counts samples, and resolve kernels are not counted in kernelLaunches.
+ * A resolved asynchronous readback resolves into a device staging buffer on the context's stream and copies
+ * from there, so the frames may be rendered into again at once.
+ *   dtr_b200_set_readback_resolve  k in 1..4 dividing width and height, else DTR_B200_ERR_ARG and the old factor
+ *                                  stays.  Applies to readbacks issued after the call.
+ *   dtr_b200_resolve_frames        flush, then write the resolved planes of frames [firstFrame, firstFrame + n)
+ *                                  into caller-owned DEVICE memory (u32 / f32 / u32 [n][H/k][W/k], each may be
+ *                                  NULL), stream-ordered on the context's stream: the zero-copy path.  ids without
+ *                                  id output (dtr_b200_set_id_output) or a bad range: DTR_B200_ERR_ARG. */
+int dtr_b200_set_readback_resolve(dtr_b200_ctx *ctx, int k);
+int dtr_b200_resolve_frames(dtr_b200_ctx *ctx, int firstFrame, int n, void *color, void *z, void *ids);
 /* Sort-first screen bands WITHOUT a gather step (SURVEY.md §8e): every rank rasterises its band
  * (dtr_b200_set_band) but writes the finished regions straight into the gathering rank's frame
  * planes over NVLink, from inside the raster kernel's write-back -- the transfer overlaps the
