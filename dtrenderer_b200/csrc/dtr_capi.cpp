@@ -791,6 +791,25 @@ int dtr_b200_set_band(dtr_b200_ctx *c, int y0, int y1)
 	return DTR_B200_OK;
 }
 
+namespace
+{
+// The nearest-texel fetch clamps u, v to [0, 1] and indexes (int)(v*h) * w + (int)(u*w) like the reference
+// (DTRendererRender.cpp:1196-1203): v == 1 lands on row h, u == 1 in the last row one texel past it.  The
+// reference reads whatever follows its bitmap there; every texture allocation carries one spare row plus one
+// texel so that the same read stays inside it (in-range results are unaffected).  After a texture with any alpha
+// below 255 the spare texels are zeros (transparent).  After an opaque one they are opaque white: a pass of
+// opaque triangles takes the deferred raster stage, which shades a visible fragment with alpha 1 and never
+// blends it, so every texel the fetch can read must be opaque for that pass to equal the single kernel; white
+// is also what an all-white texture implies, whose fetch is skipped.
+int write_texture_padding(dtr_b200_ctx *c, const TexDesc &td, bool opaque)
+{
+	const size_t               padBytes = ((size_t)td.w + 1) * 4;
+	const std::vector<uint8_t> pad(padBytes, opaque ? 0xFF : 0x00);
+	CU(cudaMemcpy(const_cast<uint32_t *>(td.texels) + (size_t)td.w * td.h, pad.data(), padBytes, cudaMemcpyHostToDevice));
+	return 0;
+}
+} // namespace
+
 int dtr_b200_upload_texture(dtr_b200_ctx *c, const uint8_t *texels, int width, int height, int bytesPerPixel, int *texId)
 {
 	if (!c || !texId) return DTR_B200_ERR_ARG;
@@ -799,14 +818,9 @@ int dtr_b200_upload_texture(dtr_b200_ctx *c, const uint8_t *texels, int width, i
 	CU(cudaSetDevice(c->device));
 	uint32_t *d     = nullptr;
 	size_t    bytes = (size_t)width * height * 4;
-	// The nearest-texel fetch clamps u, v to [0, 1] and indexes (int)(v*h) * w + (int)(u*w) like the
-	// reference (DTRendererRender.cpp:1196-1203): v == 1 lands on row h, u == 1 one texel further.  The
-	// reference reads whatever follows its bitmap there; this allocation carries one spare row plus
-	// one texel of zeros so that the same read stays inside it (in-range results are unaffected).
-	const size_t padBytes = ((size_t)width + 1) * 4;
+	const size_t padBytes = ((size_t)width + 1) * 4; // the spare texels: see write_texture_padding
 	CU(cudaMalloc((void **)&d, bytes + padBytes));
 	CU(cudaMemcpy(d, texels, bytes, cudaMemcpyHostToDevice));
-	CU(cudaMemset((uint8_t *)d + bytes, 0, padBytes));
 	c->textures.push_back(TexDesc{d, width, height});
 	{
 		// 255 * (1/255.0f) == 1.0f and 1.0f^2 == 1.0f in fp32, so an all-white opaque texture leaves
@@ -826,6 +840,8 @@ int dtr_b200_upload_texture(dtr_b200_ctx *c, const uint8_t *texels, int width, i
 		bool opaque = true;
 		for (size_t i = 3; i < bytes && opaque; i += 4) opaque = (texels[i] == 0xFF);
 		c->texIsOpaque.push_back(opaque ? 1 : 0);
+		int rc = write_texture_padding(c, c->textures.back(), opaque);
+		if (rc) return rc;
 	}
 	CU(cudaStreamSynchronize(c->stream)); // the old table may be in use
 	int rc = ensure_dev(c, c->dTextures, sizeof(TexDesc) * std::max<size_t>(c->textures.capacity(), 16));
@@ -854,6 +870,7 @@ int dtr_b200_update_texture(dtr_b200_ctx *c, int texId, const uint8_t *texels)
 	for (size_t i = 3; i < count * 4 && opaque; i += 4) opaque = (texels[i] == 0xFF);
 	c->texIsOpaque[texId] = opaque ? 1 : 0;
 	c->last.valid        = false; // a replay would keep the old "textured" decision
+	if ((rc = write_texture_padding(c, td, opaque))) return rc;
 	return DTR_B200_OK;
 }
 
