@@ -91,6 +91,8 @@ SYMBOLS = [
     ("dtr_b200_read_frames_bgr24_async", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     ("dtr_b200_set_readback_resolve", C.c_int, [C.c_void_p, C.c_int]),
     ("dtr_b200_resolve_frames", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    ("dtr_b200_create_texture", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int)]),
+    ("dtr_b200_frames_to_textures", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int)]),
     ("dtr_b200_export_frames", C.c_int, [C.c_void_p, _u8, _u8]),
     ("dtr_b200_open_peer_frames", C.c_int, [C.c_void_p, _u8, _u8]),
     ("dtr_b200_set_output_planes", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -226,6 +228,25 @@ class Renderer:
         out = np.empty(shape, np.uint8)
         self._ck(self.lib.dtr_b200_read_texture(self.ctx, tex_id, out.ctypes.data_as(_u8)))
         return out
+
+    def create_texture(self, w, h):
+        """A device-only texture of w x h texels, all zero (dtr_b200_create_texture); returns its id."""
+        tid = C.c_int(-1)
+        self._ck(self.lib.dtr_b200_create_texture(self.ctx, int(w), int(h), C.byref(tid)))
+        return tid.value
+
+    def frames_to_textures(self, first=0, n=1, tex_ids=None):
+        """Flush, then turn frames [first, first + n) into textures on the device, stream-ordered
+        (dtr_b200_frames_to_textures): frame first + i into tex_ids[i], each of out_shape.  With tex_ids None, n
+        new textures of out_shape are created.  Returns the texture ids."""
+        if tex_ids is None:
+            oh, ow = self.out_shape
+            tex_ids = [self.create_texture(ow, oh) for _ in range(n)]
+        tex_ids = [int(t) for t in tex_ids]
+        if len(tex_ids) != n:
+            raise ValueError(f"expected {n} texture ids, got {len(tex_ids)}")
+        self._ck(self.lib.dtr_b200_frames_to_textures(self.ctx, first, n, (C.c_int * n)(*tex_ids)))
+        return tex_ids
 
     def upload_mesh(self, mesh, tex_id):
         key = (id(mesh), tex_id)
@@ -522,6 +543,14 @@ class Renderer:
         t = make_transform(transform)
         self._ck(self.lib.dtr_b200_textured_triangle(self.ctx, _fp(p[0:3]), _fp(p[3:6]), _fp(p[6:9]),
                                                      _fp(uv[0:2]), _fp(uv[2:4]), _fp(uv[4:6]), tid,
+                                                     _fp(_fa(color, 4)), C.byref(t) if t else None))
+
+    def textured_triangle_id(self, p, uv, tex_id, color, transform=None):
+        """DTRRender_TexturedTriangle with a texture that is already on the device (tex_id < 0: untextured)."""
+        p, uv = _fa(p, 9), _fa(uv, 6)
+        t = make_transform(transform)
+        self._ck(self.lib.dtr_b200_textured_triangle(self.ctx, _fp(p[0:3]), _fp(p[3:6]), _fp(p[6:9]),
+                                                     _fp(uv[0:2]), _fp(uv[2:4]), _fp(uv[4:6]), int(tex_id),
                                                      _fp(_fa(color, 4)), C.byref(t) if t else None))
 
     @staticmethod

@@ -117,6 +117,7 @@ struct dtr_b200_ctx
 	std::vector<uint8_t>   texIsWhite; // every texel 0xFFFFFFFF: sampling multiplies by exactly 1.0f
 	std::vector<uint8_t>   texIsOpaque; // every texel has alpha 255: a textured fragment keeps its colour's alpha
 	DevBuf                 dTextures;
+	DevBuf                 dTexIds; // the texIds of the last dtr_b200_frames_to_textures, read by its kernel
 
 	DevBuf dCmd, dPayload;
 	// Intermediate buffers of one pass of the pipeline.  PIPE_SETS sets: a flush uses set 0; replays
@@ -725,7 +726,7 @@ void dtr_b200_destroy(dtr_b200_ctx *c)
 	for (auto &t : c->textures) cudaFree((void *)t.texels);
 	for (auto &f : c->fonts) cudaFree(f.dAtlas);
 	if (c->preStream) cudaStreamSynchronize(c->preStream);
-	std::vector<DevBuf *> bufs = {&c->dTextures, &c->dCmd, &c->dPayload};
+	std::vector<DevBuf *> bufs = {&c->dTextures, &c->dTexIds, &c->dCmd, &c->dPayload};
 	for (auto &ps : c->sets)
 	{
 		for (DevBuf *b : {&ps.prims, &ps.bounds, &ps.primZ, &ps.tileCount, &ps.tileOffset, &ps.order, &ps.lists, &ps.listBounds, &ps.listZ, &ps.segRel, &ps.primId}) bufs.push_back(b);
@@ -808,6 +809,17 @@ int write_texture_padding(dtr_b200_ctx *c, const TexDesc &td, bool opaque)
 	CU(cudaMemcpy(const_cast<uint32_t *>(td.texels) + (size_t)td.w * td.h, pad.data(), padBytes, cudaMemcpyHostToDevice));
 	return 0;
 }
+
+// Copies the texture table, with the texture just appended, to the device; *texId: the new texture's id
+int publish_new_texture(dtr_b200_ctx *c, int *texId)
+{
+	CU(cudaStreamSynchronize(c->stream)); // the old table may be in use
+	int rc = ensure_dev(c, c->dTextures, sizeof(TexDesc) * std::max<size_t>(c->textures.capacity(), 16));
+	if (rc) return rc;
+	CU(cudaMemcpy(c->dTextures.p, c->textures.data(), sizeof(TexDesc) * c->textures.size(), cudaMemcpyHostToDevice));
+	*texId = (int)c->textures.size() - 1;
+	return DTR_B200_OK;
+}
 } // namespace
 
 int dtr_b200_upload_texture(dtr_b200_ctx *c, const uint8_t *texels, int width, int height, int bytesPerPixel, int *texId)
@@ -843,12 +855,23 @@ int dtr_b200_upload_texture(dtr_b200_ctx *c, const uint8_t *texels, int width, i
 		int rc = write_texture_padding(c, c->textures.back(), opaque);
 		if (rc) return rc;
 	}
-	CU(cudaStreamSynchronize(c->stream)); // the old table may be in use
-	int rc = ensure_dev(c, c->dTextures, sizeof(TexDesc) * std::max<size_t>(c->textures.capacity(), 16));
-	if (rc) return rc;
-	CU(cudaMemcpy(c->dTextures.p, c->textures.data(), sizeof(TexDesc) * c->textures.size(), cudaMemcpyHostToDevice));
-	*texId = (int)c->textures.size() - 1;
-	return DTR_B200_OK;
+	return publish_new_texture(c, texId);
+}
+
+int dtr_b200_create_texture(dtr_b200_ctx *c, int width, int height, int *texId)
+{
+	if (!c || !texId) return DTR_B200_ERR_ARG;
+	if (width <= 0 || height <= 0 || width > 32767 || height > 32767) return fail(c, DTR_B200_ERR_ARG, "texture dimensions must be in [1,32767]");
+	CU(cudaSetDevice(c->device));
+	uint32_t    *d     = nullptr;
+	const size_t bytes = ((size_t)width * height + width + 1) * 4; // texels and the spare texels (write_texture_padding)
+	CU(cudaMalloc((void **)&d, bytes));
+	// all-zero texels: what dtr_b200_upload_texture makes of them (neither white nor opaque, zero spare texels)
+	CU(cudaMemsetAsync(d, 0, bytes, c->stream));
+	c->textures.push_back(TexDesc{d, width, height});
+	c->texIsWhite.push_back(0);
+	c->texIsOpaque.push_back(0);
+	return publish_new_texture(c, texId);
 }
 
 int dtr_b200_update_texture(dtr_b200_ctx *c, int texId, const uint8_t *texels)
@@ -890,8 +913,49 @@ int dtr_b200_read_texture(dtr_b200_ctx *c, int texId, uint8_t *rgba)
 	if (!c || !rgba) return DTR_B200_ERR_ARG;
 	if (texId < 0 || texId >= (int)c->textures.size()) return fail(c, DTR_B200_ERR_ARG, "texId out of range");
 	CU(cudaSetDevice(c->device));
+	CU(cudaStreamSynchronize(c->stream)); // dtr_b200_frames_to_textures writes texels in stream order
 	const TexDesc &td = c->textures[texId];
 	CU(cudaMemcpy(rgba, td.texels, (size_t)td.w * td.h * 4, cudaMemcpyDeviceToHost));
+	return DTR_B200_OK;
+}
+
+int dtr_b200_frames_to_textures(dtr_b200_ctx *c, int first, int n, const int *texIds)
+{
+	if (!c) return DTR_B200_ERR_ARG;
+	if (!texIds || n < 1 || !valid_frame(c, first) || !valid_frame(c, first + n - 1)) return fail(c, DTR_B200_ERR_ARG, "frame range out of bounds");
+	if (c->outColor != c->dColor)
+		return fail(c, DTR_B200_ERR_ARG, "foreign output planes are set: this context's colour planes do not hold the frames");
+	const int            ow = c->width / c->resolve, oh = c->height / c->resolve;
+	std::vector<uint8_t> taken(c->textures.size(), 0);
+	for (int i = 0; i < n; i++)
+	{
+		const int t = texIds[i];
+		if (t < 0 || t >= (int)c->textures.size()) return fail(c, DTR_B200_ERR_ARG, "texId out of range");
+		if (c->textures[t].w != ow || c->textures[t].h != oh)
+			return fail(c, DTR_B200_ERR_ARG, "texture size is not the frame size over the readback resolve factor");
+		if (taken[t]++) return fail(c, DTR_B200_ERR_ARG, "the same texId twice in one call");
+	}
+	CU(cudaSetDevice(c->device));
+	int rc = do_flush(c); // draw calls recorded so far are converted, and sample the old texels
+	if (rc) return rc;
+	if ((rc = ensure_dev(c, c->dTexIds, sizeof(int32_t) * n))) return rc;
+	CU(cudaMemcpyAsync(c->dTexIds.p, texIds, sizeof(int32_t) * n, cudaMemcpyHostToDevice, c->stream));
+	FrameTextureParams P{};
+	P.color    = c->dColor + (size_t)c->width * c->height * first;
+	P.texIds   = (const int32_t *)c->dTexIds.p;
+	P.textures = (const TexDesc *)c->dTextures.p;
+	P.width    = c->width;
+	P.height   = c->height;
+	P.frames   = n;
+	launch_frames_to_textures(P, c->resolve, c->stream);
+	CU(cudaGetLastError());
+	// the decisions draw calls take when they are recorded
+	for (int i = 0; i < n; i++)
+	{
+		c->texIsWhite[texIds[i]]  = 0;
+		c->texIsOpaque[texIds[i]] = 1;
+	}
+	c->last.valid = false; // a replay would keep the old decisions
 	return DTR_B200_OK;
 }
 

@@ -178,4 +178,14 @@ void launch_resolve_frames(const FrameResolveParams &P, int k, cudaStream_t s);
 // resolve_pack_bgr24_kernel<k, ...>: the colour of outRows output rows resolved and packed as launch_pack_bgr24 packs
 void launch_resolve_pack_bgr24(const uint32_t *color, uint32_t *out, int width, int k, size_t outRows, int pitchWords, cudaStream_t s);
 
+// Render to texture of n frames at factor k (1..4, dividing width and height): frames_to_textures_kernel<k, ...>
+struct FrameTextureParams
+{
+	const uint32_t *color;    // colour planes [frames][height][width]
+	const int32_t  *texIds;   // [frames] destination texture of each frame, (width/k) x (height/k), no two equal
+	const TexDesc  *textures; // the context's texture table
+	int             width, height, frames;
+};
+void launch_frames_to_textures(const FrameTextureParams &P, int k, cudaStream_t s);
+
 } // namespace dtr

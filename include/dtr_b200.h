@@ -239,6 +239,29 @@ int dtr_b200_read_frames_bgr24_async(dtr_b200_ctx *ctx, int firstFrame, int n, u
  *                                  id output (dtr_b200_set_id_output) or a bad range: DTR_B200_ERR_ARG. */
 int dtr_b200_set_readback_resolve(dtr_b200_ctx *ctx, int k);
 int dtr_b200_resolve_frames(dtr_b200_ctx *ctx, int firstFrame, int n, void *color, void *z, void *ids);
+/* Render to texture: frames become textures on the device, with no host round trip.  Converting frame f of a
+ * W x H context with readback resolve factor k gives a texture of (W/k) x (H/k) texels, row 0 at the bottom
+ * (frames and textures share it: no flip).  Texel (x, y) comes from w, the frame's resolved colour word at
+ * (x, y) -- the sample itself at k = 1, the resolve rule above per byte at k > 1 -- in the DTRBitmap layout:
+ * bytes R, G, B, A = (w >> 16) & 0xFF, (w >> 8) & 0xFF, w & 0xFF, 0xFF, i.e. the u32 R | G<<8 | B<<16 | 0xFF000000.
+ * The X byte is dropped; A = 255, so the texel is trivially premultiplied and the texture opaque.  Drawing with
+ * such a texture is bit for bit drawing with dtr_b200_upload_texture / dtr_b200_update_texture of the same
+ * conversion done on the host from a readback issued at that point.
+ *   dtr_b200_create_texture     a device-only texture (no host bytes, no upload), dimensions in [1, 32767].
+ *                               Its contents and flags are those of dtr_b200_upload_texture with all-zero
+ *                               texels: transparent black, neither white nor opaque.
+ *   dtr_b200_frames_to_textures flush (the conversion sees every draw call submitted before it), then write frame
+ *                               firstFrame + i into texture texIds[i] for every i < n: one kernel, stream-ordered
+ *                               on the context's stream, no host synchronisation.  Draw calls recorded afterwards
+ *                               sample the new texels; a replay needs a flush first (DTR_B200_ERR_ARG until then).
+ *                               DTR_B200_ERR_ARG, with nothing enqueued, for a bad frame range or n < 1, a texId
+ *                               out of range, a texture that is not (W/k) x (H/k), a texId given twice, or
+ *                               foreign output planes (dtr_b200_set_output_planes / dtr_b200_open_peer_frames):
+ *                               the frames are then not in this context's planes.  Like the resolve kernels the
+ *                               conversion is not counted in kernelLaunches.
+ * dtr_b200_read_texture waits for the conversions enqueued before it. */
+int dtr_b200_create_texture(dtr_b200_ctx *ctx, int width, int height, int *texId);
+int dtr_b200_frames_to_textures(dtr_b200_ctx *ctx, int firstFrame, int n, const int *texIds);
 /* Sort-first screen bands WITHOUT a gather step (SURVEY.md §8e): every rank rasterises its band
  * (dtr_b200_set_band) but writes the finished regions straight into the gathering rank's frame
  * planes over NVLink, from inside the raster kernel's write-back -- the transfer overlaps the
