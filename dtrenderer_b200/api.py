@@ -116,6 +116,8 @@ SYMBOLS = [
     ("dtr_b200_textured_triangle", C.c_int, [C.c_void_p, _f, _f, _f, _f, _f, _f, C.c_int, _f, _T]),
     ("dtr_b200_mesh", C.c_int, [C.c_void_p, C.c_int, _L, _f, _T]),
     ("dtr_b200_mesh_views", C.c_int, [C.c_void_p, C.c_int, _L, C.c_int, _f, _T, C.c_int]),
+    ("dtr_b200_triangles_device", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, _T]),
+    ("dtr_b200_mesh_views_device", C.c_int, [C.c_void_p, C.c_int, _L, C.c_int, _f, _T, C.c_int, C.c_void_p, C.c_void_p]),
     ("dtr_b200_rectangle", C.c_int, [C.c_void_p, _f, _f, _f, _T]),
     ("dtr_b200_bitmap", C.c_int, [C.c_void_p, C.c_int, _f, _T, _f]),
     ("dtr_b200_line", C.c_int, [C.c_void_p, _i32, _i32, _f]),
@@ -182,6 +184,9 @@ class Renderer:
         self._tex = {}    # id(array) -> (texId, array)
         self._mesh = {}   # (id(mesh dict), texId) -> meshId
         self._font = {}   # id(atlas) -> (fontId, font)
+        self._mesh_counts = {}  # meshId -> (numVertexes, numNormals), for the device draw calls' size checks
+        self._stream = None     # what set_stream was given (None: the context's own stream)
+        self._device_inputs = []  # tensors recorded by the device draw calls, kept alive until a flush has read them
 
     # ---- plumbing ----------------------------------------------------------------------------
     def _ck(self, rc):
@@ -192,6 +197,7 @@ class Renderer:
         if getattr(self, "ctx", None):
             self.lib.dtr_b200_destroy(self.ctx)
             self.ctx = None
+            self._device_inputs = []
 
     def __del__(self):
         try:
@@ -201,6 +207,8 @@ class Renderer:
 
     def set_stream(self, cuda_stream):
         self._ck(self.lib.dtr_b200_set_stream(self.ctx, C.c_void_p(cuda_stream)))
+        self._stream = cuda_stream or None
+        self._device_inputs = []  # (set_stream flushes)
 
     def set_band(self, y0, y1):
         self._ck(self.lib.dtr_b200_set_band(self.ctx, y0, y1))
@@ -246,6 +254,7 @@ class Renderer:
         if len(tex_ids) != n:
             raise ValueError(f"expected {n} texture ids, got {len(tex_ids)}")
         self._ck(self.lib.dtr_b200_frames_to_textures(self.ctx, first, n, (C.c_int * n)(*tex_ids)))
+        self._device_inputs = []
         return tex_ids
 
     def upload_mesh(self, mesh, tex_id):
@@ -259,6 +268,7 @@ class Renderer:
         mid = C.c_int(-1)
         self._ck(self.lib.dtr_b200_upload_mesh(self.ctx, C.byref(d), tex_id, C.byref(mid)))
         self._mesh[key] = (mid.value, mesh)
+        self._mesh_counts[mid.value] = (v.size // 4, n.size // 3)
         return mid.value
 
     def upload_mesh_faces(self, mesh, faces, arena, tex_id):
@@ -269,6 +279,7 @@ class Renderer:
                           C.c_void_p(arena.ctypes.data), arena.nbytes)
         mid = C.c_int(-1)
         self._ck(self.lib.dtr_b200_upload_mesh_faces(self.ctx, C.byref(d), tex_id, C.byref(mid)))
+        self._mesh_counts[mid.value] = (v.size // 4, n.size // 3)
         return mid.value
 
     def update_texture(self, tex_id, tex):
@@ -331,6 +342,7 @@ class Renderer:
 
     def flush(self):
         self._ck(self.lib.dtr_b200_flush(self.ctx))
+        self._device_inputs = []
 
     def replay(self):
         self._ck(self.lib.dtr_b200_replay(self.ctx))
@@ -364,6 +376,7 @@ class Renderer:
         idp = torch.empty(shape, dtype=torch.int32, device=dev) if ids else None
         self._ck(self.lib.dtr_b200_resolve_frames(self.ctx, first, n, C.c_void_p(col.data_ptr()), C.c_void_p(dep.data_ptr()),
                                                   C.c_void_p(idp.data_ptr()) if ids else None))
+        self._device_inputs = []
         self.sync()
         return (col, dep, idp) if ids else (col, dep)
 
@@ -373,23 +386,27 @@ class Renderer:
         z = z_out if z_out is not None else (np.empty(self.out_shape, np.float32) if want_z else None)
         self._ck(self.lib.dtr_b200_end_frame(self.ctx, frame, col.ctypes.data_as(C.c_void_p),
                                              z.ctypes.data_as(C.c_void_p) if z is not None else None))
+        self._device_inputs = []
         return col, z
 
     def end_frame_ptr(self, frame, color_ptr, z_ptr=None):
         """end_frame into caller-owned (e.g. pinned) host memory given as raw addresses."""
         self._ck(self.lib.dtr_b200_end_frame(self.ctx, frame, C.c_void_p(color_ptr),
                                              C.c_void_p(z_ptr) if z_ptr else None))
+        self._device_inputs = []
 
     def read_frames_ptr(self, first, n, color_ptr, z_ptr=None):
         """Flush and copy n consecutive frames into caller-owned host memory (raw addresses)."""
         self._ck(self.lib.dtr_b200_read_frames(self.ctx, first, n, C.c_void_p(color_ptr),
                                                C.c_void_p(z_ptr) if z_ptr else None))
+        self._device_inputs = []
 
     def read_frames_async_ptr(self, first, n, color_ptr, z_ptr=None):
         """Flush and enqueue the readback of n frames on the copy stream (page-locked host memory);
         returns at once.  wait_reads() blocks until every outstanding readback has landed."""
         self._ck(self.lib.dtr_b200_read_frames_async(self.ctx, first, n, C.c_void_p(color_ptr),
                                                      C.c_void_p(z_ptr) if z_ptr else None))
+        self._device_inputs = []
 
     def bgr24_pitch(self):
         """Row pitch in bytes of the 24-bit DIB rows written by read_frames_bgr24_async_ptr."""
@@ -399,6 +416,7 @@ class Renderer:
         """Flush, pack n colour planes into 24-bit bottom-up DIBs on the device and enqueue their
         readback (n * bgr24_pitch() * out_shape[0] bytes of page-locked memory); wait_reads() completes it."""
         self._ck(self.lib.dtr_b200_read_frames_bgr24_async(self.ctx, first, n, C.c_void_p(bgr_ptr)))
+        self._device_inputs = []
 
     def wait_reads(self):
         self._ck(self.lib.dtr_b200_wait_reads(self.ctx))
@@ -461,6 +479,7 @@ class Renderer:
         """Flush and read the id planes of frames [first, first + n): u32[n, H/k, W/k]."""
         out = np.empty((n, *self.out_shape), np.uint32)
         self._ck(self.lib.dtr_b200_read_ids(self.ctx, first, n, out.ctypes.data_as(C.c_void_p)))
+        self._device_inputs = []
         return out
 
     def frame_id_ptr(self, frame=0):
@@ -572,6 +591,55 @@ class Renderer:
         arr = (Transform * n)(*[make_transform(t) for t in transforms])
         self._ck(self.lib.dtr_b200_mesh_views(self.ctx, mid, C.byref(light), n, _fp(_fa(positions, 3 * n)), arr,
                                               first_frame))
+
+    # ---- draw calls from device memory (dtr_b200_triangles_device / dtr_b200_mesh_views_device) ---------------
+    def _device_tensor(self, t, n, what):
+        """Address of t, a contiguous float32 torch tensor of n elements on this renderer's device (no copy is made)."""
+        import torch
+        if not isinstance(t, torch.Tensor) or t.device != torch.device("cuda", self.device):
+            raise ValueError(f"{what} must be a torch tensor on cuda:{self.device}")
+        if t.dtype != torch.float32 or not t.is_contiguous():
+            raise ValueError(f"{what} must be contiguous float32, got {t.dtype} (contiguous: {t.is_contiguous()})")
+        if t.numel() != n:
+            raise ValueError(f"{what}: expected {n} elements, got {t.numel()}")
+        return t.data_ptr()
+
+    def _record_device(self, tensors):
+        """Order torch's work on the tensors before the flush that reads them, and keep them alive until then."""
+        import torch
+        cur = torch.cuda.current_stream(self.device)
+        if self._stream is None or cur.cuda_stream != self._stream:
+            cur.synchronize()
+        self._device_inputs.extend(t for t in tensors if t is not None)
+
+    def triangles_device(self, p, color, uv=None, tex_id=-1, transform=None):
+        """dtr_b200_triangles_device: n triangles from torch CUDA tensors p (n*9), color (n*4) and uv (n*6) or None,
+        read by the next flush; bit for bit triangles() (textured_triangle_id() per triangle with uv and tex_id >= 0)."""
+        n = p.numel() // 9 if hasattr(p, "numel") else 0
+        pp = self._device_tensor(p, 9 * n, "p")
+        cp = self._device_tensor(color, 4 * n, "color")
+        up = self._device_tensor(uv, 6 * n, "uv") if uv is not None else None
+        t = make_transform(transform)
+        self._record_device((p, color, uv))
+        self._ck(self.lib.dtr_b200_triangles_device(self.ctx, n, C.c_void_p(pp), C.c_void_p(cp),
+                                                    C.c_void_p(up) if up else None, int(tex_id), C.byref(t) if t else None))
+
+    def mesh_views_device(self, mesh_id, light_mode, light_vector, light_color, positions, transforms, vertexes,
+                          normals=None, first_frame=0):
+        """dtr_b200_mesh_views_device: view i is mesh mesh_id with vertex set i of vertexes (torch CUDA tensor of
+        n_views * numVertexes * 4 floats) and normal set i of normals (n_views * numNormals * 3, or None: the mesh's
+        own), drawn into frame first_frame + i."""
+        if mesh_id not in self._mesh_counts:
+            raise ValueError(f"mesh {mesh_id} was not uploaded through this renderer")
+        nv, nn = self._mesh_counts[mesh_id]
+        n = len(transforms)
+        vp = self._device_tensor(vertexes, n * nv * 4, "vertexes")
+        np_ = self._device_tensor(normals, n * nn * 3, "normals") if normals is not None else None
+        light = self._light(light_mode, light_vector, light_color)
+        arr = (Transform * n)(*[make_transform(t) for t in transforms])
+        self._record_device((vertexes, normals))
+        self._ck(self.lib.dtr_b200_mesh_views_device(self.ctx, mesh_id, C.byref(light), n, _fp(_fa(positions, 3 * n)), arr,
+                                                     first_frame, C.c_void_p(vp), C.c_void_p(np_) if np_ else None))
 
     def rectangle(self, mn, mx, color, transform=None):
         t = make_transform(transform)

@@ -40,7 +40,7 @@ struct MeshAsset
 {
 	float   *vertexes = nullptr, *texUV = nullptr, *normals = nullptr;
 	int32_t *faces    = nullptr;
-	uint32_t numFaces = 0;
+	uint32_t numFaces = 0, numVertexes = 0, numNormals = 0;
 	int      texId    = -1;
 };
 
@@ -51,6 +51,8 @@ struct RecItem
 	uint32_t order;      // submission order (stable sort key)
 	size_t   payload[3]; // byte offsets into the payload buffer (valid where relocate[j])
 	bool     relocate[3];
+	size_t   snap[3];    // byte offsets into the device snapshot buffer (valid where fromSnap[j]): ptr[j] read from device memory
+	bool     fromSnap[3];
 	bool     opaque;     // triangles whose every fragment has alpha 1 (colour alpha 1, no texture or an opaque one)
 };
 
@@ -111,6 +113,16 @@ struct dtr_b200_ctx
 	size_t                 payloadCap = 0, payloadUsed = 0;
 	uint8_t               *staging = nullptr; // pinned: FrameState[] + DrawItem[]
 	size_t                 stagingCap = 0;
+	// arrays of draw calls recorded from device memory (dtr_b200_triangles_device / _mesh_views_device): where they
+	// are, and where the flush's snapshot of them goes in dSnap (16-byte aligned offsets, like the payload's)
+	struct DeviceArray
+	{
+		const void *src;
+		size_t      at, bytes;
+		bool        color; // f32[n][4] triangle colours: their alphas decide the opaque stage on the device
+	};
+	std::vector<DeviceArray> devArrays;
+	size_t                   snapUsed = 0;
 
 	std::vector<MeshAsset> meshes;
 	std::vector<TexDesc>   textures;
@@ -120,6 +132,7 @@ struct dtr_b200_ctx
 	DevBuf                 dTexIds; // the texIds of the last dtr_b200_frames_to_textures, read by its kernel
 
 	DevBuf dCmd, dPayload;
+	DevBuf dSnap; // the last flush's snapshot of its device arrays (replays render from it)
 	// Intermediate buffers of one pass of the pipeline.  PIPE_SETS sets: a flush uses set 0; replays
 	// take them in turn, so that setup / scan / bin of a later replay (on preStream) run while the
 	// raster kernels of earlier replays occupy the main stream.  With THREE sets the pre-raster stages
@@ -273,25 +286,14 @@ int record_raw(dtr_b200_ctx *c, const PrimRecord &rec)
 	return 0;
 }
 
-int record_tris(dtr_b200_ctx *c, int n, const float *p, const float *color, const float *uv, int texId,
-                const dtr_b200_transform *t)
+// An ITEM_TRIS item of n triangles on the current target; the caller says where its arrays are.  opaque: the
+// texture's part of the decision (the caller adds the colours')
+RecItem &new_tris_item(dtr_b200_ctx *c, int n, int texId, const dtr_b200_transform *t)
 {
 	if (!t) t = &kDefaultTriangleTransform;
-	size_t offP, offC, offUV = 0;
-	int    rc;
-	if ((rc = payload_push(c, p, sizeof(float) * 9 * (size_t)n, &offP))) return rc;
-	if ((rc = payload_push(c, color, sizeof(float) * 4 * (size_t)n, &offC))) return rc;
-	if (uv && (rc = payload_push(c, uv, sizeof(float) * 6 * (size_t)n, &offUV))) return rc;
 	RecItem &r       = new_item(c, ITEM_TRIS, (uint32_t)c->target, (uint32_t)n);
-	r.payload[0]     = offP;
-	r.relocate[0]    = true;
-	r.payload[1]     = offC;
-	r.relocate[1]    = true;
-	r.payload[2]     = offUV;
-	r.relocate[2]    = (uv != nullptr);
 	r.item.texId     = (texId >= 0 && c->texIsWhite[texId]) ? -1 : texId;
 	r.opaque         = r.item.texId < 0 || c->texIsOpaque[r.item.texId];
-	for (int i = 0; i < n && r.opaque; i++) r.opaque = color[4 * (size_t)i + 3] == 1.0f;
 	r.item.lightMode = DTR_B200_SHADE_FULLBRIGHT; // NullRenderLightInternal (:1352-1356)
 	Basis2 b         = make_basis(t->rotation, t->scale[0], t->scale[1]);
 	r.item.xAxis[0] = b.xAxis[0]; r.item.xAxis[1] = b.xAxis[1];
@@ -299,7 +301,48 @@ int record_tris(dtr_b200_ctx *c, int n, const float *p, const float *color, cons
 	r.item.anchor[0] = t->anchor[0];
 	r.item.anchor[1] = t->anchor[1];
 	c->triangles += (uint64_t)n;
+	return r;
+}
+
+int record_tris(dtr_b200_ctx *c, int n, const float *p, const float *color, const float *uv, int texId,
+                const dtr_b200_transform *t)
+{
+	size_t offP, offC, offUV = 0;
+	int    rc;
+	if ((rc = payload_push(c, p, sizeof(float) * 9 * (size_t)n, &offP))) return rc;
+	if ((rc = payload_push(c, color, sizeof(float) * 4 * (size_t)n, &offC))) return rc;
+	if (uv && (rc = payload_push(c, uv, sizeof(float) * 6 * (size_t)n, &offUV))) return rc;
+	RecItem &r    = new_tris_item(c, n, texId, t);
+	r.payload[0]  = offP;
+	r.relocate[0] = true;
+	r.payload[1]  = offC;
+	r.relocate[1] = true;
+	r.payload[2]  = offUV;
+	r.relocate[2] = (uv != nullptr);
+	for (int i = 0; i < n && r.opaque; i++) r.opaque = color[4 * (size_t)i + 3] == 1.0f;
 	return 0;
+}
+
+// Reserves `bytes` of the flush's device snapshot for the device array src (16-byte aligned); returns the offset.
+// Nothing is read here: the flush gathers every such array with one kernel.
+size_t snap_push(dtr_b200_ctx *c, const void *src, size_t bytes, bool color)
+{
+	const size_t at = (c->snapUsed + 15) & ~(size_t)15;
+	c->devArrays.push_back({src, at, bytes, color});
+	c->snapUsed = at + bytes;
+	return at;
+}
+
+// p / color / uv of dtr_b200_triangles_device are device memory of the context's device (device or managed)
+bool on_ctx_device(const dtr_b200_ctx *c, const void *p)
+{
+	cudaPointerAttributes a{};
+	if (cudaPointerGetAttributes(&a, p) != cudaSuccess)
+	{
+		cudaGetLastError(); // (not sticky: clear it)
+		return false;
+	}
+	return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == c->device;
 }
 
 constexpr int EVENTS_PER_RUN = 7; // pre start, after setup, after scan, after bin | raster start, after the stage's first kernel, raster end
@@ -420,11 +463,14 @@ int run_pipeline(dtr_b200_ctx *c, uint32_t numActive, uint32_t numItems, uint32_
 	uint64_t total = c->last.listTotal;
 	if (!replay)
 	{
-		unsigned long long t = 0;
-		CU(cudaMemcpyAsync(&t, S.counters + 1, sizeof(t), cudaMemcpyDeviceToHost, pre));
+		// with device arrays, the gather kernel's translucent flag (counters[2]) comes back with the list total
+		unsigned long long t[2] = {0, 0};
+		const bool gathered = !c->devArrays.empty();
+		CU(cudaMemcpyAsync(t, S.counters + 1, sizeof(t[0]) * (gathered ? 2 : 1), cudaMemcpyDeviceToHost, pre));
 		CU(cudaStreamSynchronize(pre));
-		total = t;
+		total = t[0];
 		if (total >= (1ull << 31)) return fail(c, DTR_B200_ERR_OVERFLOW, "more than 2^31 (primitive, tile) pairs in one flush");
+		if (t[1]) c->last.deferred = c->last.oneKernel = false; // some device colour has alpha != 1: the pass can blend
 	}
 	if ((rc = ensure_dev(c, S.lists, sizeof(uint32_t) * (size_t)std::max<uint64_t>(total, 1)))) return rc;
 	if ((rc = ensure_dev(c, S.listBounds, 2 * sizeof(uint32_t) * (size_t)std::max<uint64_t>(total, 1)))) return rc;
@@ -545,10 +591,15 @@ int do_flush(dtr_b200_ctx *c)
 	if (totalPrims >= (1ull << 31)) return fail(c, DTR_B200_ERR_OVERFLOW, "more than 2^31 primitives in one flush");
 	const size_t numBlocks = (size_t)((totalPrims + SETUP_THREADS - 1) / SETUP_THREADS);
 	size_t   cmdBytes  = sizeof(FrameState) * numActive + sizeof(DrawItem) * numItems + sizeof(uint32_t) * numBlocks;
+	// ... | the gather kernel's segment table, one per device array (only when there are any)
+	const size_t numSegs  = c->devArrays.size();
+	const size_t segsAt   = (cmdBytes + 15) & ~(size_t)15;
+	if (numSegs) cmdBytes = segsAt + sizeof(GatherSegment) * numSegs;
 	int      rc;
 	if ((rc = ensure_pinned(c, c->staging, c->stagingCap, 0, cmdBytes))) return rc;
 	if ((rc = ensure_dev(c, c->dCmd, cmdBytes))) return rc;
 	if ((rc = ensure_dev(c, c->dPayload, std::max<size_t>(c->payloadUsed, 16)))) return rc;
+	if (numSegs && (rc = ensure_dev(c, c->dSnap, c->snapUsed))) return rc;
 
 	FrameState *fs = (FrameState *)c->staging;
 	DrawItem   *it = (DrawItem *)(c->staging + sizeof(FrameState) * numActive);
@@ -576,7 +627,10 @@ int do_flush(dtr_b200_ctx *c)
 		r.item.frame    = (uint32_t)slot;
 		r.item.primBase = (uint32_t)prim;
 		for (int j = 0; j < 3; j++)
+		{
 			if (r.relocate[j]) r.item.ptr[j] = (uint64_t)((uint8_t *)c->dPayload.p + r.payload[j]);
+			if (r.fromSnap[j]) r.item.ptr[j] = (uint64_t)((uint8_t *)c->dSnap.p + r.snap[j]);
+		}
 		it[i] = r.item;
 		prim += r.item.count;
 		if (prim >= (1ull << 31)) return fail(c, DTR_B200_ERR_OVERFLOW, "more than 2^31 primitives in one flush");
@@ -596,10 +650,35 @@ int do_flush(dtr_b200_ctx *c)
 	for (uint32_t s = 0; s < numActive; s++)
 		if (c->frames[active[s]].recorded == 0) fs[s].primBegin = fs[s].primEnd = 0;
 
+	GatherParams gather{};
+	if (numSegs)
+	{
+		GatherSegment *seg   = (GatherSegment *)(c->staging + segsAt);
+		uint64_t       chunk = 0;
+		for (size_t s = 0; s < numSegs; s++)
+		{
+			const dtr_b200_ctx::DeviceArray &a = c->devArrays[s];
+			seg[s] = GatherSegment{(uint64_t)(uintptr_t)a.src, (uint64_t)((uint8_t *)c->dSnap.p + a.at), (uint64_t)a.bytes, (uint32_t)chunk, a.color ? 1u : 0u};
+			chunk += gather_chunks(a.bytes);
+		}
+		if (chunk >= (1ull << 32)) return fail(c, DTR_B200_ERR_OVERFLOW, "more than 2^32 gather chunks of device arrays in one flush");
+		gather.segs        = (const GatherSegment *)((uint8_t *)c->dCmd.p + segsAt);
+		gather.numSegs     = (uint32_t)numSegs;
+		gather.numChunks   = (uint32_t)chunk;
+		gather.translucent = c->sets[0].counters + 2; // read back with the list total (run_pipeline)
+	}
 	c->uploadBytes = cmdBytes + c->payloadUsed;
 	CU(cudaMemcpyAsync(c->dCmd.p, c->staging, cmdBytes, cudaMemcpyHostToDevice, c->stream));
 	if (c->payloadUsed)
 		CU(cudaMemcpyAsync(c->dPayload.p, c->payload, c->payloadUsed, cudaMemcpyHostToDevice, c->stream));
+	if (numSegs)
+	{
+		// the snapshot the pipeline (and every replay of this flush) reads instead of the callers' arrays; like the
+		// readback resolve kernels it is not counted in kernelLaunches
+		CU(cudaMemsetAsync(gather.translucent, 0, sizeof(unsigned long long), c->stream));
+		launch_gather_device_inputs(gather, c->limits, c->stream);
+		CU(cudaGetLastError());
+	}
 
 	c->last.anyTextured = false;
 	for (uint32_t i = 0; i < numItems; i++) c->last.anyTextured = c->last.anyTextured || (it[i].type != ITEM_RAW && it[i].texId >= 0);
@@ -630,6 +709,8 @@ int do_flush(dtr_b200_ctx *c)
 	}
 	c->rec.clear();
 	c->payloadUsed = 0;
+	c->devArrays.clear();
+	c->snapUsed = 0;
 	return rc;
 }
 
@@ -726,7 +807,7 @@ void dtr_b200_destroy(dtr_b200_ctx *c)
 	for (auto &t : c->textures) cudaFree((void *)t.texels);
 	for (auto &f : c->fonts) cudaFree(f.dAtlas);
 	if (c->preStream) cudaStreamSynchronize(c->preStream);
-	std::vector<DevBuf *> bufs = {&c->dTextures, &c->dTexIds, &c->dCmd, &c->dPayload};
+	std::vector<DevBuf *> bufs = {&c->dTextures, &c->dTexIds, &c->dCmd, &c->dPayload, &c->dSnap};
 	for (auto &ps : c->sets)
 	{
 		for (DevBuf *b : {&ps.prims, &ps.bounds, &ps.primZ, &ps.tileCount, &ps.tileOffset, &ps.order, &ps.lists, &ps.listBounds, &ps.listZ, &ps.segRel, &ps.primId}) bufs.push_back(b);
@@ -998,8 +1079,10 @@ int dtr_b200_upload_mesh(dtr_b200_ctx *c, const dtr_b200_mesh_desc *m, int texId
 	}
 	CU(cudaSetDevice(c->device));
 	MeshAsset a;
-	a.numFaces = m->numFaces;
-	a.texId    = texId;
+	a.numFaces    = m->numFaces;
+	a.numVertexes = m->numVertexes;
+	a.numNormals  = m->numNormals;
+	a.texId       = texId;
 	int rc = upload_mesh_arrays(c, a, m->vertexes, m->numVertexes, m->texUV, m->numTexUV, m->normals, m->numNormals);
 	if (rc)
 	{
@@ -1022,8 +1105,10 @@ int dtr_b200_upload_mesh_faces(dtr_b200_ctx *c, const dtr_b200_mesh_faces_desc *
 	if (texId >= (int)c->textures.size()) return fail(c, DTR_B200_ERR_ARG, "texId out of range");
 	CU(cudaSetDevice(c->device));
 	MeshAsset a;
-	a.numFaces = m->numFaces;
-	a.texId    = texId;
+	a.numFaces    = m->numFaces;
+	a.numVertexes = m->numVertexes;
+	a.numNormals  = m->numNormals;
+	a.texId       = texId;
 	int rc = upload_mesh_arrays(c, a, m->vertexes, m->numVertexes, m->texUV, m->numTexUV, m->normals, m->numNormals);
 	uint8_t  *dFaces = nullptr, *dArena = nullptr;
 	uint32_t *dErr = nullptr, err = 0;
@@ -1808,6 +1893,59 @@ int dtr_b200_mesh_views(dtr_b200_ctx *c, int meshId, const dtr_b200_light *light
 		r.item.lightVec[2] = light->vector[2];
 		memcpy(r.item.color, light->color, sizeof(float) * 4);
 		c->triangles += m.numFaces;
+	}
+	return DTR_B200_OK;
+}
+
+int dtr_b200_triangles_device(dtr_b200_ctx *c, int n, const float *p, const float *color, const float *uv, int texId,
+                              const dtr_b200_transform *t)
+{
+	if (!c) return DTR_B200_ERR_ARG;
+	if (n <= 0 || !p || !color) return DTR_B200_OK;
+	if (texId >= (int)c->textures.size()) return fail(c, DTR_B200_ERR_ARG, "texId out of range");
+	if (!on_ctx_device(c, p) || !on_ctx_device(c, color) || (uv && !on_ctx_device(c, uv)))
+		return fail(c, DTR_B200_ERR_ARG, "p / color / uv must be device memory of the context's device");
+	RecItem &r    = new_tris_item(c, n, (uv && texId >= 0) ? texId : -1, t);
+	r.snap[0]     = snap_push(c, p, sizeof(float) * 9 * (size_t)n, false);
+	r.fromSnap[0] = true;
+	r.snap[1]     = snap_push(c, color, sizeof(float) * 4 * (size_t)n, true);
+	r.fromSnap[1] = true;
+	if (uv)
+	{
+		r.snap[2]     = snap_push(c, uv, sizeof(float) * 6 * (size_t)n, false);
+		r.fromSnap[2] = true;
+	}
+	return DTR_B200_OK;
+}
+
+int dtr_b200_mesh_views_device(dtr_b200_ctx *c, int meshId, const dtr_b200_light *light, int nViews, const float *pos,
+                               const dtr_b200_transform *transforms, int firstFrame, const float *vertexes, const float *normals)
+{
+	if (!c) return DTR_B200_ERR_ARG;
+	if (!light || !pos || !transforms || nViews <= 0 || !vertexes) return DTR_B200_OK;
+	if (meshId < 0 || meshId >= (int)c->meshes.size()) return fail(c, DTR_B200_ERR_ARG, "meshId out of range");
+	if (!valid_frame(c, firstFrame) || !valid_frame(c, firstFrame + nViews - 1))
+		return fail(c, DTR_B200_ERR_ARG, "views do not fit the context's frames");
+	if (!on_ctx_device(c, vertexes) || (normals && !on_ctx_device(c, normals)))
+		return fail(c, DTR_B200_ERR_ARG, "vertexes / normals must be device memory of the context's device");
+	const size_t first = c->rec.size();
+	int          rc    = dtr_b200_mesh_views(c, meshId, light, nViews, pos, transforms, firstFrame);
+	if (rc) return rc;
+	// view v: vertex set v (and normal set v) instead of the mesh's own arrays
+	const MeshAsset &m  = c->meshes[meshId];
+	const size_t     vB = sizeof(float) * 4 * (size_t)m.numVertexes, nB = sizeof(float) * 3 * (size_t)m.numNormals;
+	const size_t     vAt = snap_push(c, vertexes, vB * nViews, false);
+	const size_t     nAt = normals ? snap_push(c, normals, nB * nViews, false) : 0;
+	for (int v = 0; v < nViews; v++)
+	{
+		RecItem &r    = c->rec[first + v];
+		r.snap[0]     = vAt + vB * v; // vB is a multiple of 16: every set stays float4 aligned
+		r.fromSnap[0] = true;
+		if (normals)
+		{
+			r.snap[2]     = nAt + nB * v;
+			r.fromSnap[2] = true;
+		}
 	}
 	return DTR_B200_OK;
 }

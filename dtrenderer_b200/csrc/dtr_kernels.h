@@ -188,4 +188,23 @@ struct FrameTextureParams
 };
 void launch_frames_to_textures(const FrameTextureParams &P, int k, cudaStream_t s);
 
+// Snapshot of the device-resident draw-call inputs of a flush (gather_device_inputs_kernel): segment i copies
+// `bytes` (a multiple of 4) from src to dst (16-byte aligned) and covers chunks [firstChunk, next firstChunk) of
+// gather_chunks(bytes) each.  color: the segment is f32[n][4] colours whose alphas are checked.
+constexpr int      GATHER_THREADS = 256;
+constexpr uint32_t GATHER_CHUNK   = GATHER_THREADS * 64; // bytes of one segment a CTA copies per step
+struct GatherSegment
+{
+	uint64_t src, dst, bytes;
+	uint32_t firstChunk, color;
+};
+inline uint32_t gather_chunks(uint64_t bytes) { return (uint32_t)((bytes + GATHER_CHUNK - 1) / GATHER_CHUNK); }
+struct GatherParams
+{
+	const GatherSegment *segs; // [numSegs], firstChunk ascending
+	uint32_t             numSegs, numChunks;
+	unsigned long long  *translucent; // set to 1 when some colour alpha is not 1.0f; zeroed by the host
+};
+void launch_gather_device_inputs(const GatherParams &P, const LaunchLimits &L, cudaStream_t s);
+
 } // namespace dtr

@@ -169,8 +169,9 @@ typedef struct dtr_b200_mesh_faces_desc
 	size_t                    arenaBytes;
 } dtr_b200_mesh_faces_desc;
 int dtr_b200_upload_mesh_faces(dtr_b200_ctx *ctx, const dtr_b200_mesh_faces_desc *mesh, int texId, int *meshId);
-/* Forget cached device copies after the host changed an asset in place: the texture / mesh keeps its
- * id, its contents are uploaded again (same dimensions / counts required). */
+/* Forget cached device copies after the host changed a texture in place: the texture keeps its id, its
+ * contents are uploaded again (same dimensions required).  A mesh's vertexes and normals can change per draw
+ * call instead, from device memory: dtr_b200_mesh_views_device. */
 int dtr_b200_update_texture(dtr_b200_ctx *ctx, int texId, const uint8_t *texels);
 
 /* ---- frame -------------------------------------------------------------------------------- */
@@ -373,6 +374,33 @@ int dtr_b200_mesh(dtr_b200_ctx *ctx, int meshId, const dtr_b200_light *light, co
  * parallel batch): pos f32[nViews*3], transforms[nViews]. */
 int dtr_b200_mesh_views(dtr_b200_ctx *ctx, int meshId, const dtr_b200_light *light, int nViews,
                         const float *pos, const dtr_b200_transform *transforms, int firstFrame);
+/* Draw calls whose arrays live in DEVICE memory of the context's device (device or managed allocations, e.g. torch
+ * CUDA tensors): geometry made on the GPU is drawn without a round trip over the host link.
+ *   dtr_b200_triangles_device   n triangles: p f32[n*9], color f32[n*4], uv f32[n*6] or NULL; texId < 0 or uv == NULL:
+ *                               untextured.  Same meaning, transform handling, triangle ids and counters as
+ *                               dtr_b200_triangles (and, when textured, dtr_b200_textured_triangle per triangle).
+ *   dtr_b200_mesh_views_device  dtr_b200_mesh_views with per-view vertex sets: vertexes f32[nViews][numVertexes][4]
+ *                               (w must be 1, as for dtr_b200_upload_mesh), normals f32[nViews][numNormals][3] or NULL
+ *                               (the mesh's own normals); texUV, faces and texture come from the uploaded mesh.  View i
+ *                               is mesh meshId with vertex set i, drawn into frame firstFrame + i.
+ * Equivalence: drawing with these calls is bit for bit drawing the same values through dtr_b200_triangles /
+ * dtr_b200_textured_triangle, or through dtr_b200_mesh_views on a mesh uploaded with those vertexes and normals --
+ * colour, depth, ids, setPixels, triangles and the opaque stage that runs (dtr_b200_last_pass_deferred).  Only
+ * uploadBytes differs: the arrays never cross the host link.
+ * When the arrays are read: on the context's stream, by the flush that executes the call (any entry that flushes).
+ * Whatever writes them must be ordered before that flush on that stream.  Once that flush returns the library no
+ * longer reads them (a flush waits on the host for its list total): the caller may then free or overwrite them.
+ * Replay: dtr_b200_replay renders what that flush read, from the library's own device snapshot; it never re-reads
+ * the caller's arrays.
+ * Errors: DTR_B200_ERR_ARG, with nothing recorded, for a pointer that cudaPointerGetAttributes does not report as
+ * device or managed memory of the context's device (host memory, pinned or not, included), and for meshId, texId or
+ * the frame range out of range.  n <= 0 or NULL p / color / vertexes (or light / pos / transforms) return
+ * DTR_B200_OK without drawing.  The arrays need no particular alignment. */
+int dtr_b200_triangles_device(dtr_b200_ctx *ctx, int n, const float *p, const float *color, const float *uv,
+                              int texId, const dtr_b200_transform *transform);
+int dtr_b200_mesh_views_device(dtr_b200_ctx *ctx, int meshId, const dtr_b200_light *light, int nViews,
+                               const float *pos, const dtr_b200_transform *transforms, int firstFrame,
+                               const float *vertexes, const float *normals);
 int dtr_b200_rectangle(dtr_b200_ctx *ctx, const float min[2], const float max[2],
                        const float color[4], const dtr_b200_transform *transform);
 int dtr_b200_bitmap(dtr_b200_ctx *ctx, int texId, const float pos[2],
